@@ -2,7 +2,7 @@
 """bench.py -- ray-samples/s of the per-ray rendering hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--workload black_800|black_400|cfg1|fern_high|train_dtu] [--shard images|rays]
+                    [--workload black_800|black_400|cfg1|fern_high|train_dtu] [--shard images|rays] [--dump-outputs DIR]
 
 Headline (default flags): a "step" renders ONE full synthetic query image through the hot path (sample_depth -> coarse
 pass -> fused resampling -> fine pass), encoder outputs given.  Workload `black_800` = the geometry BASELINE.json's metric
@@ -21,6 +21,11 @@ Other BASELINE.json configurations (selectable as the main line with --workload,
              output key gathered in one NCCL all-gather) = strong scaling; the collective is timed separately
   train_dtu  cfg5: one optimisation step per rank on 512 rays of a DTU-shape scene (8 views 304x400), native backward,
              flat-bucket gradient all-reduce (timed separately), Adam = weak scaling
+
+--dump-outputs DIR writes what the headline's device-resident arm rendered in its last timed step (rank 0), one
+DIR/<key>.npy per output key in float32 (float64 for integer keys), at most 64 MB in all: a larger output keeps the same
+seeded sample of rays in every key (DIR/ray_index.npy).  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 
 --impl reference times the UNMODIFIED reference's own implementation of the path (baseline/_ref, the verbatim copy made by
 baseline/install_ref.py: NeuralRayBaseRenderer.render_impl over the chunk loop of renderer.py:237-254, encoder outputs
@@ -633,6 +638,27 @@ def init_net_bench(dr, dev, reps, timed):
 
 # ---- headline -----------------------------------------------------------------------------------------------------------------
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out, rays, path):
+    """Writes a render's output dict as path/<key>.npy (float32; float64 for integer keys).  Keys are [1, rays, ...]; when
+    they come to more than DUMP_BYTES, every key keeps the same rays, a sorted sample drawn with a fixed seed."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    per_ray = sum(v[0, 0].numel() * (8 if v.dtype in (torch.int32, torch.int64) else 4) for v in out.values())
+    idx = None
+    if per_ray * rays > DUMP_BYTES:
+        keep = DUMP_BYTES // per_ray
+        idx = torch.randperm(rays, generator=torch.Generator().manual_seed(0))[:keep].sort()[0]
+        np.save(os.path.join(path, "ray_index.npy"), idx.numpy().astype(np.float64))
+    for k, v in out.items():
+        assert v.shape[:2] == (1, rays), (k, tuple(v.shape))
+        v = v.detach()[:, idx.to(v.device)] if idx is not None else v.detach()
+        v = v.cpu().numpy()
+        np.save(os.path.join(path, k + ".npy"), v.astype(np.float64 if v.dtype.kind in "iu" else np.float32))
+
+
 def run_headline(ctx, args):
     from neuray_b200 import _lib
     rank, world, dev = ctx.rank, ctx.world, ctx.dev
@@ -673,7 +699,10 @@ def run_headline(ctx, args):
     # ---- device-resident arm (value) with per-kernel event timing of the two kernels of a pass ----
     dq = {k: v.to(dev) for k, v in que.items()}
     dr = {k: v.to(dev) for k, v in ref.items()}
-    step_resident = lambda: step_device(dict(dq), dr)      # the per-frame map repack runs inside every render() call
+    last = {}
+
+    def step_resident():                  # the per-frame map repack runs inside every render() call
+        last["out"] = step_device(dict(dq), dr)
 
     sampler = ClockSampler(ctx.local)
     for _ in range(args.warmup):
@@ -715,6 +744,8 @@ def run_headline(ctx, args):
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(last["out"], rays, args.dump_outputs)
 
     peaks, peaks_src = {}, "fallback"
     pth = os.path.join(ROOT, "MEASURED_PEAKS.json")
@@ -832,7 +863,13 @@ def main():
     ap.add_argument("--ref-rays", type=int, default=512, help="rays per step for --impl reference")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-aux", action="store_true", help="skip the auxiliary legs (fern_high sharded, train_dtu, eager GPU baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's outputs of its last timed step as DIR/<key>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload in ("fern_high", "train_dtu")):
+        ap.error("--dump-outputs writes the headline's outputs: --impl b200 with black_800, black_400 or cfg1")
     if args.impl == "reference":
         if args.workload in ("fern_high", "train_dtu"):
             args.workload = "fern_high" if args.workload == "fern_high" else "black_800"

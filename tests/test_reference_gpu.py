@@ -1,105 +1,56 @@
-"""GPU: the drop-in proof.  The UNMODIFIED reference (baseline/_ref, the verbatim copy made by baseline/install_ref.py; or
-/root/reference in the build container) is imported, its own NeuralRayGenRenderer is built and run under CUDA twice -- as
-is, and after neuray_b200.patch.install() -- on the same seeded inputs, and everything the reference's callers read is
-compared: every output key of forward() in eval and training mode, and after backward() of the reference's kind of loss
-(render + depth terms, self-hit-prob term) the gradient of EVERY parameter of the network (hot-path modules, image
-encoder, vis encoder, init net) -- i.e. also what flows out of the CUDA path into the PyTorch encoders in front of it.
+"""GPU: the drop-in proof.  The UNMODIFIED reference's own NeuralRayGenRenderer, render_ops and losses were run on seeded inputs
+(oracle/gen_golden_dropin.py -> tests/golden/dropin_*.npz); the native path runs on the same inputs and parameters, and
+everything the reference's callers read is compared with what the reference computed: every output key of forward() in eval
+mode (gen_depth and gen_cost_volume models, init net and encoders included), and in training mode every output key, the
+gradient of every hot-path parameter and the gradients the path hands to the encoders in front of it, after backward() of the
+reference's kind of loss (render + depth terms, self-hit-prob term).
+
+The encoders and the init net have no native backward: in training patch.install() keeps the reference's own PyTorch modules
+in front of the path.  So the training comparison feeds the path the reference's encoder outputs and checks what flows back
+into them; the encoders' backward, the reference's code, is linear in that gradient.
 
 This is the test of SURVEY.md section 8b: `render.py` / `run_training.py` construct the network by name, call
 `network(data)` and `loss.backward()`; nothing else touches the renderer.
 """
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
 
-import ref_import
-from neuray_b200 import patch, synthetic
+import gen_golden_dropin as gd
+from neuray_b200 import renderer, synthetic
 
 pytestmark = pytest.mark.gpu
 
-
-@pytest.fixture(autouse=True)
-def fp32_convolutions():
-    """cuDNN runs fp32 convolutions through TF32 by default; the encoders in front of the path would then turn a 1e-6
-    difference in the feature-map gradients into a 1e-2 difference of their own weight gradients (sums with heavy
-    cancellation), which says nothing about the path under test."""
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cudnn.deterministic, torch.backends.cudnn.benchmark)
-    torch.backends.cudnn.allow_tf32 = False
-    # one fixed cuDNN algorithm per convolution: otherwise the heuristics may pick different ones in the two runs (the choice
-    # depends on the free workspace memory), and the encoders' own outputs already differ by 1e-5 between two runs of the
-    # UNMODIFIED reference -- which their ill-conditioned backward turns into 1e-2 (tools/debug_initnet.py)
-    torch.backends.cudnn.deterministic, torch.backends.cudnn.benchmark = True, False
-    yield
-    torch.backends.cudnn.allow_tf32, torch.backends.cudnn.deterministic, torch.backends.cudnn.benchmark = old
-
-DN = 24
-CFG = {"init_net_type": "depth", "use_hierarchical_sampling": True, "use_depth_loss": True, "dist_decoder_cfg": {"use_vis": False},
-       "depth_sample_num": DN, "fine_depth_sample_num": DN, "agg_net_cfg": {"sample_num": DN}, "fine_agg_net_cfg": {"sample_num": DN},
-       "ray_batch_num": 192, "render_depth": True, "depth_loss_coords_num": 256}
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+CFG = gd.CFG
 
 
-@pytest.fixture(scope="module")
-def ref_mod():
-    if not ref_import.available():
-        pytest.skip("the reference tree is missing: run `python baseline/install_ref.py` (or __graft_entry__.build()) before gpurun; "
-                    "baseline/_ref travels to the box with the snapshot")
-    mod = ref_import.load_reference()
-    yield mod
-    patch.uninstall()
+def golden(name, prefix=""):
+    z = np.load(os.path.join(GOLDEN, name))
+    return {k[len(prefix):]: torch.from_numpy(z[k]) for k in z.files if k.startswith(prefix) and z[k].dtype.kind != "U"}
 
 
-def _smooth(rs, shape, lo, hi, cells=8):
-    """Low-frequency random field (bilinear upsampling of a coarse grid): images and depth maps of real scenes are smooth at
-    the pixel scale; white noise would make every bilinear lookup hypersensitive to the last bit of its coordinates."""
-    n, c, h, w = shape
-    coarse = torch.from_numpy(rs.uniform(lo, hi, (n, c, max(2, h // cells), max(2, w // cells))).astype(np.float32))
-    return torch.nn.functional.interpolate(coarse, size=(h, w), mode="bilinear", align_corners=True)
+def gen_net(cfg, tag):
+    """The native NeuralRayGenFrameRenderer with the parameters the reference ran with (same state-dict names and shapes)."""
+    shapes = json.loads(str(np.load(os.path.join(GOLDEN, "dropin_eval.npz"))[f"{tag}_shapes"]))
+    net = renderer.NeuralRayGenFrameRenderer(cfg)
+    assert gd.front_shapes(net) == shapes
+    missing, unexpected = net.load_state_dict(gd.weights(cfg, shapes), strict=False)
+    assert not unexpected and all("imagenet_" in k for k in missing), (missing, unexpected)
+    return net.cuda().eval()
 
 
-def make_data(rfn=6, rays=384, self_feats=False, seed=3):
-    que, ref = synthetic.make_scene(64, 80, rfn, seed=seed, smooth=2)
-    ref = dict(ref)
-    ref.pop("ray_feats"), ref.pop("img_feats")
-    rs = np.random.RandomState(seed)
-    ref["imgs"] = _smooth(rs, tuple(ref["imgs"].shape), 0.0, 1.0)
-    que = dict(que, imgs=_smooth(rs, tuple(que["imgs"].shape), 0.0, 1.0))
-    ref["depth"] = _smooth(rs, (rfn, 1, 64, 80), 2.5, 5.0)
-    ref["true_depth"] = ref["depth"]
-    n = que["coords"].shape[1]
-    idx = torch.from_numpy(rs.permutation(n)[:rays])
-    que = dict(que, coords=que["coords"][:, idx].contiguous())
-    if self_feats:
-        que["ray_feats"] = torch.from_numpy(rs.standard_normal((1, 32, 16, 20)).astype(np.float32))
-    return que, ref
-
-
-def build(ref_mod, cfg, seed=0):
-    torch.manual_seed(seed)
-    net = ref_mod.NeuralRayGenRenderer(cfg)
-    # hot-path modules: random init with a density head that terminates rays gradually (the default head of make_weights
-    # multiplies the last density layer by 8, which also multiplies fp32 summation-order noise between cuBLAS and the kernels)
-    W = synthetic.make_weights(cfg, seed=seed, sigma_gain=1.0, sigma_bias=0.02)
-    missing, unexpected = net.load_state_dict(W, strict=False)
-    assert not unexpected
-    return net.cuda()
-
-
-def run(net, que, ref, is_train, seed=77):
+def run(net, que, ref, is_train, src=None):
     data = {"que_imgs_info": synthetic.to_device(que, "cuda"), "ref_imgs_info": synthetic.to_device(ref, "cuda")}
+    if src is not None:
+        data["src_imgs_info"] = synthetic.to_device(src, "cuda")
     if not is_train:
         data["eval"] = True
-    torch.manual_seed(seed)            # randperm of the depth-loss coordinates, torch.rand of the fine quantiles
+    torch.manual_seed(gd.FORWARD_SEED)            # randperm of the depth-loss coordinates, torch.rand of the fine quantiles
     return net(data)
-
-
-def loss_of(out):
-    """The shape of the reference's training loss (network/loss.py:46-132): render terms on both passes + a depth term on
-    the decoder means + the self-hit-prob consistency term when present."""
-    loss = ((out["pixel_colors_nr"] - out["pixel_colors_gt"]) ** 2).mean() + ((out["pixel_colors_nr_fine"] - out["pixel_colors_gt_fine"]) ** 2).mean()
-    loss = loss + 0.1 * out["depth_mean"].abs().mean() + 0.1 * out["depth_mean_fine"].abs().mean()
-    if "hit_prob_self" in out:
-        loss = loss + ((out["hit_prob_self"] - out["hit_prob_nr"].detach()) ** 2).mean() + ((out["hit_prob_self_fine"] - out["hit_prob_nr_fine"].detach()) ** 2).mean()
-    return loss
 
 
 def compare_outputs(a, b, fine_bad_frac):
@@ -116,129 +67,78 @@ def compare_outputs(a, b, fine_bad_frac):
         assert bad <= allowed, (k, bad, float((x - y).abs().max()))
 
 
-def test_eval_forward_patched_equals_unpatched(ref_mod):
-    que, ref = make_data()
-    net = build(ref_mod, CFG).eval()
+def test_eval_forward_patched_equals_unpatched():
+    que, ref = gd.make_data()
+    net = gen_net(CFG, "depth")
     with torch.no_grad():
-        want = run(net, que, ref, False)
-        patch.install()
-        try:
-            got = run(net, que, ref, False)
-        finally:
-            patch.uninstall()
+        got = run(net, que, ref, False)
     torch.cuda.synchronize()
     assert "hit_prob_nr" not in got and "depth_mean_fine" in got
-    compare_outputs(got, want, fine_bad_frac=0.01)
-
-
-class GradTap:
-    """Captures (and optionally perturbs) the gradients that flow OUT of the rendering path into the encoders in front of it:
-    d loss / d output of every image_encoder / vis_encoder call (the path's inputs img_feats / ray_feats)."""
-
-    def __init__(self, net, inject=None):
-        self.grads, self.inject, self.handles = [], inject, []
-        for name in ("image_encoder", "vis_encoder"):
-            self.handles.append(getattr(net, name).register_forward_hook(self._fwd(name)))
-
-    def _fwd(self, name):
-        def hook(module, inputs, output):
-            idx = len(self.grads)
-            self.grads.append(None)
-
-            def on_grad(g):
-                self.grads[idx] = (name, g.detach().clone())
-                if self.inject is not None:     # replace what arrives here by a given gradient (see the test below)
-                    return g + self.inject[idx]
-            output.register_hook(on_grad)
-        return hook
-
-    def close(self):
-        for h in self.handles:
-            h.remove()
+    compare_outputs(got, golden("dropin_eval.npz", "depth_out_"), fine_bad_frac=0.01)
 
 
 @pytest.mark.parametrize("self_hit", [False, True])
-def test_training_forward_and_every_gradient(ref_mod, self_hit):
-    """forward() in training mode + backward() of the reference's kind of loss, unpatched vs patched:
+def test_training_forward_and_every_gradient(self_hit):
+    """forward() in training mode + backward() of the reference's kind of loss, native path against the reference:
       * every output key;
-      * every parameter of the hot-path modules (dist_decoder, agg_net and their fine twins), directly;
-      * the gradients the path hands to the encoders in front of it (d ray_feats, d img_feats), directly;
-      * every parameter upstream of the path (image encoder, vis encoder, init net).  The encoders' backward is the
-        reference's own PyTorch code in both runs and LINEAR in the gradient it receives, so their parameter gradients must be
-        exactly what that backward makes of the path's output gradients: the reference is run once more with the measured
-        difference of the feature-map gradients (patched - reference, 1e-5 .. 2e-4 of the maps' largest entry: last-bit
-        differences of the fine-pass sample positions) added where the path hands them over, and every upstream parameter
-        gradient of the patched network has to agree with that run to fp32 accuracy.  (Comparing them with the plain reference
-        run instead would test the conditioning of ~20 convolution + InstanceNorm layers, which turn a 1e-4 difference into
-        1e-2: tools/debug_ref_grads.py.)"""
+      * every parameter of the hot-path modules (dist_decoder, agg_net and their fine twins);
+      * the gradients the path hands to the encoders in front of it (d img_feats, d ray_feats of the reference views and, with
+        the self-hit term, d ray_feats of the query)."""
     cfg = dict(CFG, use_self_hit_prob=self_hit)
-    que, ref = make_data(self_feats=self_hit)
-    net = build(ref_mod, cfg).train()
-    grads, outs, taps = {}, {}, {}
-
-    def run_mode(mode, inject=None):
-        tap = GradTap(net, inject)
-        if mode == "patched":
-            patch.install()
-        try:
-            net.zero_grad(set_to_none=True)
-            out = run(net, que, ref, True)
-            loss_of(out).backward()
-            torch.cuda.synchronize()
-        finally:
-            patch.uninstall()
-            tap.close()
-        outs[mode] = {k: v.detach().clone() for k, v in out.items()}
-        grads[mode] = {k: (p.grad.detach().clone() if p.grad is not None else None) for k, p in net.named_parameters()}
-        taps[mode] = tap.grads
-
-    run_mode("reference")
-    run_mode("patched")
-    compare_outputs(outs["patched"], outs["reference"], fine_bad_frac=0.01)
+    name = f"dropin_train_self_hit_{int(self_hit)}"
+    que, ref = gd.make_data(self_feats=self_hit)
+    net = renderer.NeuralRayRenderPath(cfg)
+    net.load_state_dict(gd.weights(cfg, {}), strict=True)
+    net.cuda().train()
+    feats = {k: v.cuda().requires_grad_(True) for k, v in golden(name + "_inputs.npz").items()}
+    dq, dr = synthetic.to_device(que, "cuda"), synthetic.to_device(ref, "cuda")
+    dr["img_feats"], dr["ray_feats"] = feats["ref_img_feats"], feats["ref_ray_feats"]
+    if self_hit:
+        dq["ray_feats"] = feats["que_ray_feats"]
+    torch.manual_seed(gd.FORWARD_SEED)
+    out = net.render(dq, dr, True)
+    out.update(net.predict_mean_for_depth_loss(dr))      # NeuralRayGenRenderer.forward with use_depth_loss and a true depth
+    gd.loss_of(out).backward()
+    torch.cuda.synchronize()
+    compare_outputs(out, golden(name + ".npz", "out_"), fine_bad_frac=0.01)
     # what the path hands upstream
-    assert len(taps["patched"]) == len(taps["reference"]) >= 2
-    delta = []
-    for (name, g_ref), (_, g) in zip(taps["reference"], taps["patched"]):
+    for k, g_ref in golden(name + ".npz", "feat_grad_").items():
+        g = feats[k].grad.cpu()
         rel = float((g - g_ref).abs().max()) / float(g_ref.abs().max())
-        delta.append(g - g_ref)
-        print(f"d loss / d {name} output: relative difference {rel:.2e}")
-        assert rel <= 2e-3, (name, rel)
-    run_mode("reference_plus_delta", inject=delta)    # the reference's backward fed with the patched path's output gradients
+        print(f"d loss / d {k}: relative difference {rel:.2e}")
+        assert rel <= 2e-3, (k, rel)
+    grads = golden(name + ".npz", "grad_")
+    params = dict(net.named_parameters())
+    assert set(grads) <= set(params), set(grads) - set(params)
+    for k, p in params.items():           # no gradient in the reference (the fine vis decoder without the self-hit term)
+        if k not in grads:
+            assert p.grad is None or float(p.grad.abs().max()) < 1e-7, k
     module_scale = {}
-    for k, g_ref in grads["reference"].items():
-        if g_ref is not None:
-            m = k.split(".")[0]
-            module_scale[m] = max(module_scale.get(m, 0.0), float(g_ref.abs().max()))
-    checked, flows_upstream, worst = 0, 0, (0.0, "")
-    for k, g_ref in grads["reference"].items():
-        g = grads["patched"][k]
-        if g_ref is None or float(g_ref.abs().max()) == 0.0:
-            assert g is None or float(g.abs().max()) < 1e-7, k
-            continue
-        assert g is not None, f"{k}: the patched network sends no gradient here"
+    for k, g_ref in grads.items():
+        m = k.split(".")[0]
+        module_scale[m] = max(module_scale.get(m, 0.0), float(g_ref.abs().max()))
+    checked, worst = 0, (0.0, "")
+    for k, g_ref in grads.items():
+        assert params[k].grad is not None, f"{k}: the native path sends no gradient here"
+        g = params[k].grad.cpu()
         scale = float(g_ref.abs().max())
-        err = float((g - g_ref).abs().max())
-        # parameters whose true gradient is zero (a conv bias in front of an InstanceNorm, the bias in front of a softmax) hold
-        # rounding noise only, in the reference too: measured against the module's largest gradient entry
+        if scale == 0.0:
+            assert float(g.abs().max()) < 1e-7, k
+            continue
+        # parameters whose true gradient is zero (the bias in front of a softmax) hold rounding noise only, in the reference
+        # too: measured against the module's largest gradient entry
         noise = 1e-4 * module_scale[k.split(".")[0]]
-        upstream = k.split(".")[0] in ("image_encoder", "vis_encoder", "init_net")
-        if upstream:
-            # 2e-2: init_net additionally sees its own inputs through the CUDA get_diff_feats (1e-6-level differences of the
-            # reprojection features), and its backward runs through ~20 convolution + InstanceNorm layers (tools/debug_initnet2.py)
-            err = float((g - grads["reference_plus_delta"][k]).abs().max())
-            assert err <= 2e-2 * scale + noise, (k, err, scale, noise)
-        else:
-            # 5e-3: the fine pass runs on resampled depths that differ in the last bits between the two implementations
-            assert err <= 5e-3 * scale + noise, (k, err, scale, noise)
+        err = float((g - g_ref).abs().max())
+        # 5e-3: the fine pass runs on resampled depths that differ in the last bits between the two implementations
+        assert err <= 5e-3 * scale + noise, (k, err, scale, noise)
         if scale > noise:
             worst = max(worst, (err / scale, k))
         checked += 1
-        flows_upstream += upstream
-    print(f"worst relative gradient difference {worst[0]:.2e} ({worst[1]}), {checked} parameters, {flows_upstream} upstream of the path")
-    assert checked > 250 and flows_upstream > 100, (checked, flows_upstream)
+    print(f"worst relative gradient difference {worst[0]:.2e} ({worst[1]}), {checked} parameters")
+    assert checked > 100, checked
 
 
-def test_render_ops_refuse_to_cut_a_graph(ref_mod):
+def test_render_ops_refuse_to_cut_a_graph():
     """A drop-in without a backward raises when handed an input that requires grad (instead of silently detaching)."""
     from neuray_b200 import _lib, render_ops
     d = torch.rand(1, 8, 16, device="cuda", requires_grad=True)
@@ -246,97 +146,40 @@ def test_render_ops_refuse_to_cut_a_graph(ref_mod):
         render_ops.depth2dists(d)
     with torch.no_grad():
         render_ops.depth2dists(d)
-    fm = torch.randn(2, 32, 12, 16, device="cuda", requires_grad=True)
-    pts = torch.rand(2, 50, 2, device="cuda") * torch.tensor([60.0, 44.0], device="cuda")
-    mask = (torch.rand(2, 50, device="cuda") > 0.2).float()
+    fm, pts, mask = (t.cuda() for t in gd.interpolation_inputs())
+    fm.requires_grad_(True)
     out = render_ops.interpolate_feature_map(fm, pts, mask, 48, 64)
     out.square().sum().backward()
-    import network.render_ops as ref_ops          # the reference's own torch implementation
-    fm2 = fm.detach().clone().requires_grad_(True)
-    want = ref_ops.interpolate_feature_map(fm2, pts, mask, 48, 64)
-    want.square().sum().backward()
-    assert torch.allclose(out, want, atol=1e-5) and torch.allclose(fm.grad, fm2.grad, atol=1e-4, rtol=1e-4)
+    want = golden("dropin_eval.npz")                     # the reference's own torch implementation
+    assert torch.allclose(out.cpu(), want["interp_out"], atol=1e-5)
+    assert torch.allclose(fm.grad.cpu(), want["interp_grad"], atol=1e-4, rtol=1e-4)
 
 
-def test_losses_patched_equal_unpatched(ref_mod):
-    """network.loss.name2loss (what train/trainer.py builds its losses from) before and after patch.install(): the three
-    losses on the outputs of one training-mode forward of the reference network, values and the gradients with respect to
-    every output tensor they read."""
-    import network.loss as ref_loss
-    cfg = dict(CFG, use_self_hit_prob=True)
-    que, ref = make_data(self_feats=True)
-    net = build(ref_mod, cfg).train()
-    with torch.no_grad():
-        out = run(net, que, ref, True)
-    dref = synthetic.to_device(ref, "cuda")
-    data_gt = {"ref_imgs_info": dref, "scene_name": "dtu_train/scan1"}
-    reads = ("pixel_colors_nr", "pixel_colors_nr_fine", "depth_mean", "depth_mean_fine", "hit_prob_self", "hit_prob_self_fine")
-    cfgs = {"render": {"use_nr_fine_loss": True}, "depth": {"depth_loss_type": "smooth_l1"}, "consist": {}}
-
-    def evaluate():
-        data_pr = {k: (v.detach().clone().requires_grad_(True) if k in reads else v) for k, v in out.items()}
-        res = {}
-        for name, c in cfgs.items():
-            res.update(ref_loss.name2loss[name](c)(data_pr, data_gt, 0))
-        total = sum((i + 1.0) * v.sum() for i, v in enumerate(res.values()))
-        total.backward()
-        return {k: v.detach() for k, v in res.items()}, {k: data_pr[k].grad for k in reads}
-
-    want, gwant = evaluate()
-    patch.install()
-    try:
-        from neuray_b200 import losses
-        assert ref_loss.name2loss["depth"] is losses.DepthLoss
-        got, ggot = evaluate()
-    finally:
-        patch.uninstall()
-    assert ref_loss.name2loss["depth"] is not losses.DepthLoss
+def test_losses_patched_equal_unpatched():
+    """network.loss.name2loss (what train/trainer.py builds its losses from) against the native losses that patch.install()
+    puts in its place: the three losses on the outputs of one training-mode forward of the reference network, values and the
+    gradients with respect to every output tensor they read."""
+    from neuray_b200 import losses
+    _, ref = gd.make_data(self_feats=True)
+    out = {k: v.cuda() for k, v in golden("dropin_eval.npz", "loss_in_").items()}
+    got, ggot = gd.evaluate_losses(losses.name2loss, out, synthetic.to_device(ref, "cuda"))
+    want, gwant = golden("dropin_eval.npz", "loss_val_"), golden("dropin_eval.npz", "loss_grad_")
     assert set(got) == set(want) == {"loss_rgb_nr", "loss_rgb_nr_fine", "loss_depth", "loss_depth_fine", "loss_prob", "loss_prob_fine"}
     for k in want:
-        assert torch.allclose(got[k], want[k], rtol=2e-5, atol=1e-6), (k, got[k], want[k])
-    for k in reads:
+        assert torch.allclose(got[k].cpu(), want[k], rtol=2e-5, atol=1e-6), (k, got[k], want[k])
+    for k in gd.LOSS_READS:
         assert gwant[k] is not None and ggot[k] is not None, k
-        err, scale = float((ggot[k] - gwant[k]).abs().max()), float(gwant[k].abs().max())
+        err, scale = float((ggot[k].cpu() - gwant[k]).abs().max()), float(gwant[k].abs().max())
         assert err <= 1e-4 * scale + 1e-9, (k, err, scale)
 
 
-def test_cost_volume_model_eval_forward_patched_equals_unpatched(ref_mod):
-    """The neuray_gen_cost_volume model (init_net_type 'cost_volume': CostVolumeInitNet with its frozen MVSNet, random-init here) in
-    eval mode, as is and after patch.install(): the patched run goes through nr_mvsnet_fwd + nr_cost_volume_head_fwd, the native
-    encoders and the render kernels."""
-    import os
+def test_cost_volume_model_eval_forward_patched_equals_unpatched():
+    """The neuray_gen_cost_volume model (init_net_type 'cost_volume': CostVolumeInitNet with its MVSNet, seeded here) in eval
+    mode: the native run goes through nr_mvsnet_fwd + nr_cost_volume_head_fwd, the native encoders and the render kernels."""
     cfg = dict(CFG, init_net_type="cost_volume")
-    que, ref = synthetic.make_scene(64, 96, 4, seed=5, smooth=2)
-    _, src = synthetic.make_scene(64, 96, 3, seed=6, smooth=2)
-    ref = dict(ref)
-    ref.pop("ray_feats"), ref.pop("img_feats")
-    rs = np.random.RandomState(5)
-    ref["imgs"] = _smooth(rs, tuple(ref["imgs"].shape), 0.0, 1.0)
-    src = {"imgs": _smooth(rs, tuple(src["imgs"].shape), 0.0, 1.0), "poses": src["poses"], "Ks": src["Ks"]}
-    ref["nn_ids"] = torch.from_numpy(np.stack([rs.permutation(3)[:2] for _ in range(4)]).astype(np.int64))
-    que = dict(que, imgs=_smooth(rs, tuple(que["imgs"].shape), 0.0, 1.0), coords=que["coords"][:, torch.from_numpy(rs.permutation(que["coords"].shape[1])[:384])].contiguous())
-    cwd = os.getcwd()
-    os.chdir(ref_import.REFERENCE_ROOT)          # CostVolumeInitNet opens network/mvsnet/mvsnet_pl.ckpt relative to the reference root
-    try:
-        net = build(ref_mod, cfg).eval()
-    finally:
-        os.chdir(cwd)
-    # soften the cost volume's logits so that the depth softmax is not an argmax (random-init / foreign-data weights saturate it)
+    que, ref, src = gd.cost_volume_data()
+    net = gen_net(cfg, "cv")
     with torch.no_grad():
-        net.init_net.mvsnet.cost_regularization.prob.weight.mul_(0.05)
-
-    def go():
-        data = {"que_imgs_info": synthetic.to_device(que, "cuda"), "ref_imgs_info": synthetic.to_device(ref, "cuda"),
-                "src_imgs_info": synthetic.to_device(src, "cuda"), "eval": True}
-        torch.manual_seed(7)
-        return net(data)
-
-    with torch.no_grad():
-        want = go()
-        patch.install()
-        try:
-            got = go()
-        finally:
-            patch.uninstall()
+        got = run(net, que, ref, False, src)
     torch.cuda.synchronize()
-    compare_outputs(got, want, fine_bad_frac=0.01)
+    compare_outputs(got, golden("dropin_eval.npz", "cv_out_"), fine_bad_frac=0.01)

@@ -1,4 +1,7 @@
 """GPU: every stand-alone render_ops drop-in against the oracle's restatement of the same reference function."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
@@ -74,16 +77,14 @@ def test_compositing_and_resampling(scene):
     fd_o = orc.sample_fine_depth(depth, hit, que["depth_range"], 16, False)
     fd_g = render_ops.sample_fine_depth(depth.cuda(), hit.cuda(), que["depth_range"].cuda(), 16, False)
     close(fd_g, fd_o, atol=2e-5, what="sample_fine_depth")
-    # inv_mode=False (render_ops.py:182,224): resampling directly in depth; pinned to the unmodified reference where it is present
+    # inv_mode=False (render_ops.py:182,224): resampling directly in depth; both modes pinned to the unmodified reference's
+    # results on these inputs (oracle/gen_golden_dropin.py)
     fd_o2 = orc.sample_fine_depth(depth, hit, que["depth_range"], 16, False, inv_mode=False)
     fd_g2 = render_ops.sample_fine_depth(depth.cuda(), hit.cuda(), que["depth_range"].cuda(), 16, False, inv_mode=False)
     close(fd_g2, fd_o2, atol=2e-5, what="sample_fine_depth inv_mode=False")
-    import ref_import
-    if ref_import.available():
-        ref_import.load_reference()
-        import network.render_ops as ref_ops
-        close(fd_o2, ref_ops.sample_fine_depth(depth, hit, que["depth_range"], 16, False, inv_mode=False), atol=1e-6, what="oracle vs reference, inv_mode=False")
-        close(fd_o, ref_ops.sample_fine_depth(depth, hit, que["depth_range"], 16, False), atol=1e-5, what="oracle vs reference, inv_mode=True")
+    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dropin_eval.npz"))
+    close(fd_o2, torch.from_numpy(z["fine_depth_lin"]), atol=1e-6, what="oracle vs reference, inv_mode=False")
+    close(fd_o, torch.from_numpy(z["fine_depth_inv"]), atol=1e-5, what="oracle vs reference, inv_mode=True")
 
 
 def test_interpolation_backward_matches_the_oracle_autograd(scene):
