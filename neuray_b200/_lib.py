@@ -187,11 +187,6 @@ LAUNCHES = 0
 PROFILE = None
 
 
-def count_launches(n):
-    global LAUNCHES
-    LAUNCHES += n
-
-
 class NeurayB200Error(RuntimeError):
     pass
 
@@ -259,3 +254,37 @@ def on_device(t):
     if not t.is_cuda:
         raise NeurayB200Error("neuray_b200 ops need CUDA tensors (no CPU fallback)")
     return torch.cuda.device(t.device)
+
+
+def call(name, *args, on, kernels=1, stream=None, what=None):
+    """Enqueues the library entry point `name`(*args, stream) on the device of tensor `on`.  The stream is the current
+    stream of that device unless `stream` is given (a backward that must follow the stream its forward ran on).  Raises
+    NeurayB200Error on a nonzero return and adds `kernels`, the number of kernels the entry point launches, to LAUNCHES."""
+    global LAUNCHES
+    with on_device(on):
+        check(getattr(lib(), name)(*args, stream_of(on) if stream is None else stream), what or name)
+    LAUNCHES += kernels
+
+
+def f32(t):
+    """t as a contiguous fp32 tensor outside autograd (t itself, detached, when it already is one)."""
+    return t.detach().contiguous().float()
+
+
+# Grow-only device workspaces, reused across passes, chunks and frames.  The C-ABI never allocates (the caller owns the
+# workspace); taking hundreds of MB of point records and tapes per pass from torch's caching allocator every time fragmented
+# it and cost cudaMalloc calls in steady state.  Work is stream-ordered on the caller's stream; using one buffer from
+# several streams at once is not supported.  Each key is its own buffer: buffers whose keys differ can be live together.
+_WORKSPACES = {}
+
+
+def workspace(key, numel, dev, dtype):
+    """The first `numel` elements of the (key, dev) workspace, grown (never shrunk) to fit."""
+    import torch
+    k = (key, str(dev))
+    buf = _WORKSPACES.get(k)
+    if buf is None or buf.numel() < numel:
+        buf = None                     # the old buffer is freed before the larger one is allocated
+        _WORKSPACES.pop(k, None)
+        buf = _WORKSPACES[k] = torch.empty(numel, dtype=dtype, device=dev)
+    return buf[:numel]

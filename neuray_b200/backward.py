@@ -10,18 +10,6 @@ import torch
 from . import _lib
 
 HEADS = ("mean_decoder", "var_decoder", "aw_decoder", "vis_decoder")
-_WS = {}
-
-
-def _ws(key, numel, dev):
-    buf = _WS.get((key, str(dev)))
-    if buf is None or buf.numel() < numel:
-        _WS.pop((key, str(dev)), None)
-        buf = torch.empty(numel, dtype=torch.float32, device=dev)
-        _WS[(key, str(dev))] = buf
-    return buf[:numel]
-
-
 TILE = 128
 
 
@@ -142,9 +130,8 @@ def assemble_param_grads_fused(names, dec, agg, n_heads, tape_row, grad_row, tap
         _DESC_CACHE[key] = hit
     table, descs, offs, total = hit
     out = torch.zeros(total, dtype=torch.float32, device=tape_row.device)
-    _lib.check(_lib.lib().nr_tape_gemms(descs, len(table), _lib.ptr(tape_row), _lib.ptr(grad_row), rows, _lib.ptr(tape_point),
-                                        _lib.ptr(grad_point), points, _lib.ptr(out), stream), "nr_tape_gemms")
-    _lib.count_launches(1)
+    _lib.call("nr_tape_gemms", descs, len(table), _lib.ptr(tape_row), _lib.ptr(grad_row), rows, _lib.ptr(tape_point), _lib.ptr(grad_point), points,
+              _lib.ptr(out), on=out, stream=stream)
     blocks = [out[o:o + t[2] * (t[5] + 1)].view(t[2], t[5] + 1) for o, t in zip(offs, table)]
     return _finish(names, table, blocks)
 
@@ -160,16 +147,15 @@ def render_pass_backward(p, names, dec, agg, g_pix, g_hit, g_depth, want_feat_gr
     dev = (g_pix if g_pix is not None else g_hit if g_hit is not None else g_depth).device
     n_points = p.rn * p.dn
     shapes = tape_shapes(p.rfn, n_points)
-    bufs = {k: _ws(k, sh[0] * sh[1] * sh[2], dev).view(sh) for k, sh in shapes.items()}
+    bufs = {k: _lib.workspace(k, sh[0] * sh[1] * sh[2], dev, torch.float32).view(sh) for k, sh in shapes.items()}
     d_feat = torch.zeros(feat_shape, dtype=torch.float32, device=dev) if want_feat_grads else None
     b = _lib.NrBwdParams()
-    keep = [t.contiguous().float() if t is not None else None for t in (g_pix, g_hit, g_depth)]
+    keep = [_lib.f32(t) if t is not None else None for t in (g_pix, g_hit, g_depth)]
     b.d_pixel_colors, b.d_hit_prob, b.d_render_depth = (_lib.ptr(t) for t in keep)
     b.tape_row, b.grad_row = _lib.ptr(bufs["tape_row"]), _lib.ptr(bufs["grad_row"])
     b.tape_point, b.grad_point = _lib.ptr(bufs["tape_point"]), _lib.ptr(bufs["grad_point"])
     b.d_feat = _lib.ptr(d_feat)
-    _lib.check(_lib.lib().nr_render_pass_bwd(C.byref(p), C.byref(b), stream), "nr_render_pass_bwd")
-    _lib.count_launches(11)
+    _lib.call("nr_render_pass_bwd", C.byref(p), C.byref(b), on=bufs["tape_row"], stream=stream, kernels=11)
     grads = assemble_param_grads_fused(names, dec, agg, 4 if p.use_vis else 3, bufs["tape_row"], bufs["grad_row"], bufs["tape_point"],
                                        bufs["grad_point"], p.rfn * n_points, n_points, stream)
     if d_feat is None:
@@ -216,9 +202,7 @@ class RenderPassFn(torch.autograd.Function):
             return (None, None, None, None, *[None] * len(params))
         p, _keep, feat_shape, stream = ctx.bwd
         want_feat = ray_feats.requires_grad or img_feats.requires_grad
-        with _lib.on_device(ray_feats):
-            grads, drf, dimf = render_pass_backward(p, meta["names"], meta["dec"], meta["agg"], g_pix, g_hit, g_depth, want_feat,
-                                                    feat_shape, stream)
+        grads, drf, dimf = render_pass_backward(p, meta["names"], meta["dec"], meta["agg"], g_pix, g_hit, g_depth, want_feat, feat_shape, stream)
         gp = [grads[n] if t.requires_grad else None for n, t in zip(meta["names"], params)]
         return (None, None, drf if ray_feats.requires_grad else None, dimf if img_feats.requires_grad else None, *gp)
 
@@ -231,9 +215,7 @@ class SelfHitProbFn(torch.autograd.Function):
         p = meta["params"]()
         hit = torch.empty(p.rn, p.dn, dtype=torch.float32, device=que_ray_feats.device)
         p.hit = _lib.ptr(hit)
-        with _lib.on_device(que_ray_feats):
-            _lib.check(_lib.lib().nr_self_hit_prob(C.byref(p), meta["stream"]), "nr_self_hit_prob")
-        _lib.count_launches(1)
+        _lib.call("nr_self_hit_prob", C.byref(p), on=que_ray_feats, stream=meta["stream"])
         ctx.meta = meta
         ctx.feats_need = que_ray_feats.requires_grad
         ctx.need = [t.requires_grad for t in dec_params]
@@ -245,14 +227,12 @@ class SelfHitProbFn(torch.autograd.Function):
         index_map = meta["index_map"]
         p = meta["params"]()
         dev = g_hit.device
-        g = g_hit[0].contiguous().float()
+        g = _lib.f32(g_hit[0])
         hit = torch.empty(p.rn, p.dn, dtype=torch.float32, device=dev)
         d_w = torch.zeros(index_map[0].numel(), dtype=torch.float32, device=dev)
         d_map = torch.zeros(meta["map_shape"], dtype=torch.float32, device=dev) if ctx.feats_need else None
         p.hit, p.d_hit, p.d_w_point, p.d_map = _lib.ptr(hit), _lib.ptr(g), _lib.ptr(d_w), _lib.ptr(d_map)
-        with _lib.on_device(g_hit):
-            _lib.check(_lib.lib().nr_self_hit_prob(C.byref(p), meta["stream"]), "nr_self_hit_prob (backward)")
-        _lib.count_launches(1)
+        _lib.call("nr_self_hit_prob", C.byref(p), on=g_hit, stream=meta["stream"], what="nr_self_hit_prob (backward)")
         grads = unpack_point_grads(index_map, d_w)
         gp = [grads[n] if need else None for n, need in zip(meta["dec_names"], ctx.need)]
         return (None, d_map[None] if d_map is not None else None, *gp)

@@ -15,11 +15,12 @@ is False and `renderer.render` keeps calling the owner's own torch modules (the 
 There is no CPU path: CUDA tensors only.
 """
 import ctypes as C
+import functools
 
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, weights
 
 
 def unet_param_names(blocks):
@@ -136,43 +137,13 @@ def set_precision(mode):
         raise ValueError(f"encoder precision {mode!r}: 'fp32' or 'tf32'")
     PRECISION = mode
 
-_WS = {}
 
-
-def _workspace(key, nbytes, dev):
-    buf = _WS.get((key, str(dev)))
-    if buf is None or buf.numel() < nbytes:
-        _WS.pop((key, str(dev)), None)
-        buf = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        _WS[(key, str(dev))] = buf
-    return buf
-
-
-def _packed(module, names, which, dev):
-    """Packed parameter buffer of an encoder (nr_*_encoder_pack), cached on the module, re-packed when a parameter changed."""
-    sd = dict(module.named_parameters())
-    missing = [n for n in names if n not in sd]
-    if missing:
-        raise _lib.NeurayB200Error(f"{which} encoder: parameters {missing[:3]}... not found (expected the reference's state-dict names)")
-    params = [sd[n] for n in names]
-    stamp = tuple((p.data_ptr(), p._version) for p in params) + (str(dev),)
-    hit = module.__dict__.get("_nr_enc_pack")
-    if hit is None or hit[0] != stamp:
-        if params[0].device != torch.device(dev):
-            raise _lib.NeurayB200Error(f"{which} encoder parameters live on {params[0].device} but the images are on {dev}")
-        lay = _lib.NrEncoderLayout()
-        _lib.check(_lib.lib().nr_encoder_layout(C.byref(lay)), "nr_encoder_layout")
-        n_floats = {"image": lay.image_packed_floats, "vis": lay.vis_packed_floats, "depth_init": lay.depth_init_packed_floats}[which]
-        keep = [p.detach().contiguous().float() for p in params]
-        ptrs = (C.c_void_p * len(keep))(*[t.data_ptr() for t in keep])
-        out = torch.empty(n_floats, dtype=torch.float32, device=dev)
-        fn = {"image": _lib.lib().nr_image_encoder_pack, "vis": _lib.lib().nr_vis_encoder_pack, "depth_init": _lib.lib().nr_depth_init_pack}[which]
-        with torch.cuda.device(dev):
-            _lib.check(fn(ptrs, len(keep), _lib.ptr(out), torch.cuda.current_stream(dev).cuda_stream), f"nr_{which}_pack")
-        _lib.count_launches(1)
-        hit = (stamp, out)
-        module.__dict__["_nr_enc_pack"] = hit
-    return hit[1]
+@functools.cache
+def layout():
+    """nr_encoder_layout: tensor counts and packed sizes of the image encoder, the vis encoder and DepthInitNet."""
+    lay = _lib.NrEncoderLayout()
+    _lib.check(_lib.lib().nr_encoder_layout(C.byref(lay)), "nr_encoder_layout")
+    return lay
 
 
 def image_dims(h, w):
@@ -189,14 +160,12 @@ def image_encoder_into(module, imgs, out, out_off):
     if c != 3:
         raise _lib.NeurayB200Error(f"image_encoder expects [n,3,h,w] images, got {tuple(imgs.shape)}")
     dev = imgs.device
-    packed = _packed(module, image_param_names(), "image", dev)
+    packed = weights.packed(module, "image", image_param_names(), "nr_image_encoder_pack", layout().image_packed_floats, dev)
     nbytes = _lib.lib().nr_image_encoder_workspace(n, h, w)
-    ws = _workspace("image", nbytes, dev)
-    x = imgs.detach().contiguous().float()
-    with _lib.on_device(imgs):
-        _lib.check(_lib.lib().nr_image_encoder_fwd(_lib.ptr(packed), _lib.ptr(x), n, h, w, _lib.ptr(out), out.shape[-1], out_off, int(PRECISION == "tf32"),
-                                                   ws.data_ptr(), nbytes, _lib.stream_of(imgs)), "nr_image_encoder_fwd")
-    _lib.count_launches(IMAGE_LAUNCHES)
+    ws = _lib.workspace("image", nbytes, dev, torch.uint8)
+    x = _lib.f32(imgs)
+    _lib.call("nr_image_encoder_fwd", _lib.ptr(packed), _lib.ptr(x), n, h, w, _lib.ptr(out), out.shape[-1], out_off, int(PRECISION == "tf32"),
+              ws.data_ptr(), nbytes, on=imgs, kernels=IMAGE_LAUNCHES)
     return out
 
 
@@ -206,32 +175,26 @@ def vis_encoder_inplace(module, feat):
     if c != 64 or not feat.is_contiguous():
         raise _lib.NeurayB200Error("vis_encoder works on the contiguous [n,fh,fw,64] frame pack")
     dev = feat.device
-    packed = _packed(module, vis_param_names(), "vis", dev)
+    packed = weights.packed(module, "vis", vis_param_names(), "nr_vis_encoder_pack", layout().vis_packed_floats, dev)
     nbytes = _lib.lib().nr_vis_encoder_workspace(n, fh, fw)
-    ws = _workspace("vis", nbytes, dev)
-    with _lib.on_device(feat):
-        _lib.check(_lib.lib().nr_vis_encoder_fwd(_lib.ptr(packed), _lib.ptr(feat), n, fh, fw, int(PRECISION == "tf32"), ws.data_ptr(), nbytes, _lib.stream_of(feat)),
-                   "nr_vis_encoder_fwd")
-    _lib.count_launches(VIS_LAUNCHES)
+    ws = _lib.workspace("vis", nbytes, dev, torch.uint8)
+    _lib.call("nr_vis_encoder_fwd", _lib.ptr(packed), _lib.ptr(feat), n, fh, fw, int(PRECISION == "tf32"), ws.data_ptr(), nbytes,
+              on=feat, kernels=VIS_LAUNCHES)
     return feat
 
 
 def to_channel_last(x, out, out_off):
     """[n,c,h,w] -> channels [out_off, out_off + c) of out [n,h,w,C]."""
     n, c, h, w = x.shape
-    xx = x.detach().contiguous().float()
-    with _lib.on_device(x):
-        _lib.check(_lib.lib().nr_nchw_to_nhwc(_lib.ptr(xx), n, c, h, w, _lib.ptr(out), out.shape[-1], out_off, _lib.stream_of(x)), "nr_nchw_to_nhwc")
-    _lib.count_launches(1)
+    xx = _lib.f32(x)
+    _lib.call("nr_nchw_to_nhwc", _lib.ptr(xx), n, c, h, w, _lib.ptr(out), out.shape[-1], out_off, on=x)
 
 
 def from_channel_last(buf, off, c):
     """channels [off, off + c) of buf [n,h,w,C] -> a new [n,c,h,w] tensor (the layout the reference's callers expect)."""
     n, h, w, C_ = buf.shape
     out = torch.empty(n, c, h, w, dtype=torch.float32, device=buf.device)
-    with _lib.on_device(buf):
-        _lib.check(_lib.lib().nr_nhwc_to_nchw(_lib.ptr(buf), n, c, h, w, C_, off, _lib.ptr(out), _lib.stream_of(buf)), "nr_nhwc_to_nchw")
-    _lib.count_launches(1)
+    _lib.call("nr_nhwc_to_nchw", _lib.ptr(buf), n, c, h, w, C_, off, _lib.ptr(out), on=buf)
     return out
 
 
@@ -271,7 +234,7 @@ class VisEncoder(nn.Module):
 
 
 def _refuse_training(module):
-    if torch.is_grad_enabled() and any(p.requires_grad for p in module.parameters()):
+    if weights.wants_grad(module):
         raise _lib.NeurayB200Error(f"{type(module).__name__}: the native encoders are forward-only; run them under torch.no_grad() "
                                    "(training keeps the torch encoders upstream of the boundary)")
 
@@ -287,11 +250,9 @@ def usable(owner, ref_imgs_info):
         from . import init_nets
         if getattr(owner, "init_net", None) is None or not init_nets.init_usable(owner.init_net, ref_imgs_info):
             return False
-    if torch.is_grad_enabled() and (any(p.requires_grad for p in ie.parameters()) or any(p.requires_grad for p in ve.parameters())
-                                    or (rf is not None and rf.requires_grad)):
+    if weights.wants_grad(ie, ve) or (torch.is_grad_enabled() and rf is not None and rf.requires_grad):
         return False
-    have_i, have_v = dict(ie.named_parameters()), dict(ve.named_parameters())
-    return all(n in have_i for n in image_param_names()) and all(n in have_v for n in vis_param_names())
+    return weights.has_names(ie, image_param_names()) and weights.has_names(ve, vis_param_names())
 
 
 def encode_frame(owner, ref_imgs_info, feat):

@@ -12,11 +12,12 @@ vis encoder expects the init net's ray_feats.  `patch.install()` puts `forward_o
 forward: with a gradient wanted through the net (training) the reference's own torch code runs.  CUDA tensors only.
 """
 import ctypes as C
+import functools
 
 import torch
 import torch.nn as nn
 
-from . import _lib, encoders, init_ops
+from . import _lib, encoders, init_ops, weights
 
 BLOCKS = (2, 2, 2)
 LAUNCHES = 3 + 2 + 3 * (5 + 4) + 2 + 8 + 2 + 1 + 1 + 1       # input assembly, first layer, 3 stages, decoder, out_conv, depth_skip, conv_out
@@ -42,23 +43,16 @@ def dims(h, w):
 
 
 def usable(module, ref_imgs_info):
-    if not ref_imgs_info["imgs"].is_cuda:
-        return False
-    have = dict(module.named_parameters())
-    if not all(n in have for n in param_names()):
-        return False
-    return not (torch.is_grad_enabled() and any(p.requires_grad for p in module.parameters()))
+    return ref_imgs_info["imgs"].is_cuda and weights.has_names(module, param_names()) and not weights.wants_grad(module)
 
 
 def extract_depth_for_init(ref_imgs_info):
     """init_net.py:76-79 -> [rfn,1,h,w] normalised inverse depth."""
     depth, rng = ref_imgs_info["depth"], ref_imgs_info["depth_range"]
     rfn, _, h, w = depth.shape
-    d, r = depth.detach().contiguous().float(), rng.detach().contiguous().float()
+    d, r = _lib.f32(depth), _lib.f32(rng)
     out = torch.empty_like(d)
-    with _lib.on_device(depth):
-        _lib.check(_lib.lib().nr_extract_depth(_lib.ptr(d), _lib.ptr(r), rfn, h, w, _lib.ptr(out), _lib.stream_of(depth)), "nr_extract_depth")
-    _lib.count_launches(1)
+    _lib.call("nr_extract_depth", _lib.ptr(d), _lib.ptr(r), rfn, h, w, _lib.ptr(out), on=depth)
     return out
 
 
@@ -71,15 +65,12 @@ def forward_into(module, ref_imgs_info, out, out_off):
     dev = imgs.device
     depth = extract_depth_for_init(ref_imgs_info)
     diff = init_ops.get_diff_feats(ref_imgs_info, depth)
-    packed = encoders._packed(module, param_names(), "depth_init", dev)
+    packed = weights.packed(module, "depth_init", param_names(), "nr_depth_init_pack", encoders.layout().depth_init_packed_floats, dev)
     nbytes = _lib.lib().nr_depth_init_workspace(rfn, h, w)
-    ws = encoders._workspace("depth_init", nbytes, dev)
-    x = imgs.detach().contiguous().float()
-    with _lib.on_device(imgs):
-        _lib.check(_lib.lib().nr_depth_init_fwd(_lib.ptr(packed), _lib.ptr(x), _lib.ptr(depth), _lib.ptr(diff.contiguous()), rfn, h, w, _lib.ptr(out),
-                                                out.shape[-1], out_off, int(encoders.PRECISION == "tf32"), ws.data_ptr(), nbytes,
-                                                _lib.stream_of(imgs)), "nr_depth_init_fwd")
-    _lib.count_launches(LAUNCHES)
+    ws = _lib.workspace("depth_init", nbytes, dev, torch.uint8)
+    x = _lib.f32(imgs)
+    _lib.call("nr_depth_init_fwd", _lib.ptr(packed), _lib.ptr(x), _lib.ptr(depth), _lib.ptr(diff.contiguous()), rfn, h, w, _lib.ptr(out),
+              out.shape[-1], out_off, int(encoders.PRECISION == "tf32"), ws.data_ptr(), nbytes, on=imgs, kernels=LAUNCHES)
     return out
 
 
@@ -174,51 +165,21 @@ def _cost_volume_head_shapes(sn):
     return {n: s[n] for n in cost_volume_head_names()}
 
 
-def _named_tensors(module):
-    d = dict(module.named_parameters())
-    d.update(dict(module.named_buffers()))
-    return d
-
-
-def _packed_cv(module, which, sn, dev):
-    """Packed MVSNet ('mvsnet': BatchNorm folded, conv weights re-laid) or head parameters, cached on the module."""
-    names = ["mvsnet." + n for n in mvsnet_tensor_names()] if which == "mvsnet" else cost_volume_head_names()
-    have = _named_tensors(module)
-    missing = [n for n in names if n not in have]
-    if missing:
-        raise _lib.NeurayB200Error(f"CostVolumeInitNet: tensors {missing[:3]}... not found (expected the reference's state-dict names)")
-    tensors = [have[n] for n in names]
-    stamp = tuple((t.data_ptr(), t._version) for t in tensors) + (str(dev), sn)
-    cache = module.__dict__.setdefault("_nr_cv_pack", {})
-    hit = cache.get(which)
-    if hit is None or hit[0] != stamp:
-        n_t, n_f = C.c_int(), C.c_longlong()
-        if which == "mvsnet":
-            _lib.check(_lib.lib().nr_mvsnet_layout(C.byref(n_t), C.byref(n_f)), "nr_mvsnet_layout")
-        else:
-            _lib.check(_lib.lib().nr_cost_volume_head_layout(sn, C.byref(n_t), C.byref(n_f)), "nr_cost_volume_head_layout")
-        keep = [t.detach().contiguous().float() for t in tensors]
-        ptrs = (C.c_void_p * len(keep))(*[t.data_ptr() for t in keep])
-        out = torch.empty(n_f.value, dtype=torch.float32, device=dev)
-        st = torch.cuda.current_stream(dev).cuda_stream
-        with torch.cuda.device(dev):
-            if which == "mvsnet":
-                _lib.check(_lib.lib().nr_mvsnet_pack(ptrs, len(keep), _lib.ptr(out), st), "nr_mvsnet_pack")
-            else:
-                _lib.check(_lib.lib().nr_cost_volume_head_pack(sn, ptrs, len(keep), _lib.ptr(out), st), "nr_cost_volume_head_pack")
-        _lib.count_launches(1)
-        hit = (stamp, out)
-        cache[which] = hit
-    return hit[1]
+@functools.cache
+def _packed_floats(which, sn):
+    """Size of the packed MVSNet ('mvsnet': BatchNorm folded, conv weights re-laid) or cost-volume head ('head') buffer."""
+    n_t, n_f = C.c_int(), C.c_longlong()
+    if which == "mvsnet":
+        _lib.check(_lib.lib().nr_mvsnet_layout(C.byref(n_t), C.byref(n_f)), "nr_mvsnet_layout")
+    else:
+        _lib.check(_lib.lib().nr_cost_volume_head_layout(sn, C.byref(n_t), C.byref(n_f)), "nr_cost_volume_head_layout")
+    return n_f.value
 
 
 def cost_volume_usable(module, ref_imgs_info, src_imgs_info):
     if src_imgs_info is None or not ref_imgs_info["imgs"].is_cuda or "nn_ids" not in ref_imgs_info:
         return False
-    have = _named_tensors(module)
-    if not all(("mvsnet." + n) in have for n in mvsnet_tensor_names()) or not all(n in have for n in cost_volume_head_names()):
-        return False
-    return not (torch.is_grad_enabled() and any(p.requires_grad for p in module.parameters()))
+    return weights.has_names(module, ["mvsnet." + n for n in mvsnet_tensor_names()] + cost_volume_head_names()) and not weights.wants_grad(module)
 
 
 def mvsnet_cost_volume(module, ref_imgs_info, src_imgs_info, is_train):
@@ -227,10 +188,9 @@ def mvsnet_cost_volume(module, ref_imgs_info, src_imgs_info, is_train):
     rfn, _, h, w = imgs.shape
     dev = imgs.device
     sn = int(module.cfg["cost_volume_sn"])
-    packed = _packed_cv(module, "mvsnet", sn, dev)
-    f = lambda t: t.detach().contiguous().float()
-    keep = [f(imgs), f(simgs), f(ref_imgs_info["Ks"]), f(ref_imgs_info["poses"]), f(src_imgs_info["Ks"]), f(src_imgs_info["poses"]),
-            f(ref_imgs_info["depth_range"]), ref_imgs_info["nn_ids"].detach().to(torch.int32).contiguous()]
+    packed = weights.packed(module, "mvsnet", ["mvsnet." + n for n in mvsnet_tensor_names()], "nr_mvsnet_pack", _packed_floats("mvsnet", sn), dev)
+    keep = [_lib.f32(t) for t in (imgs, simgs, ref_imgs_info["Ks"], ref_imgs_info["poses"], src_imgs_info["Ks"], src_imgs_info["poses"],
+                                  ref_imgs_info["depth_range"])] + [ref_imgs_info["nn_ids"].detach().to(torch.int32).contiguous()]
     a = _lib.NrMvsIn()
     (a.ref_imgs, a.src_imgs, a.ref_Ks, a.ref_poses, a.src_Ks, a.src_poses, a.depth_range, a.nn_ids) = [_lib.ptr(t) for t in keep[:7]] + [keep[7].data_ptr()]
     a.rfn, a.sn, a.nn, a.h, a.w, a.dn, a.is_train = rfn, simgs.shape[0], keep[7].shape[1], h, w, sn, int(bool(is_train))
@@ -239,13 +199,11 @@ def mvsnet_cost_volume(module, ref_imgs_info, src_imgs_info, is_train):
     nbytes = _lib.lib().nr_mvsnet_workspace(C.byref(a))
     if nbytes <= 0:
         raise _lib.NeurayB200Error(f"MVSNet: unsupported shape (images {h}x{w}, {sn} depth planes: h/4, w/4 and the planes must be multiples of 8)")
-    ws = encoders._workspace("mvsnet", nbytes, dev)
+    ws = _lib.workspace("mvsnet", nbytes, dev, torch.uint8)
     prob = torch.empty(rfn, ho.value, wo.value, sn, dtype=torch.float32, device=dev)
     depth = torch.empty(rfn, ho.value, wo.value, dtype=torch.float32, device=dev)
-    with _lib.on_device(imgs):
-        _lib.check(_lib.lib().nr_mvsnet_fwd(_lib.ptr(packed), C.byref(a), _lib.ptr(prob), _lib.ptr(depth), ws.data_ptr(), nbytes, _lib.stream_of(imgs)),
-                   "nr_mvsnet_fwd")
-    _lib.count_launches(2 + 8 * (rfn + simgs.shape[0]) + 1 + rfn * 13)
+    _lib.call("nr_mvsnet_fwd", _lib.ptr(packed), C.byref(a), _lib.ptr(prob), _lib.ptr(depth), ws.data_ptr(), nbytes, on=imgs,
+              kernels=2 + 8 * (rfn + simgs.shape[0]) + 1 + rfn * 13)
     return prob, depth
 
 
@@ -257,15 +215,13 @@ def cost_volume_forward_into(module, ref_imgs_info, src_imgs_info, is_train, out
     sn = int(module.cfg["cost_volume_sn"])
     prob, depth = mvsnet_cost_volume(module, ref_imgs_info, src_imgs_info, is_train)
     depth_norm = extract_depth_for_init({"depth": depth[:, None], "depth_range": ref_imgs_info["depth_range"]})
-    packed = _packed_cv(module, "head", sn, dev)
+    packed = weights.packed(module, "head", cost_volume_head_names(), "nr_cost_volume_head_pack", _packed_floats("head", sn), dev, sn)
     nbytes = _lib.lib().nr_cost_volume_head_workspace(sn, rfn, h, w)
-    ws = encoders._workspace("cv_head", nbytes, dev)
-    x = imgs.detach().contiguous().float()
-    with _lib.on_device(imgs):
-        _lib.check(_lib.lib().nr_cost_volume_head_fwd(sn, _lib.ptr(packed), _lib.ptr(x), _lib.ptr(prob), _lib.ptr(depth_norm), rfn, h, w, _lib.ptr(out),
-                                                      out.shape[-1], out_off, int(encoders.PRECISION == "tf32"), ws.data_ptr(), nbytes,
-                                                      _lib.stream_of(imgs)), "nr_cost_volume_head_fwd")
-    _lib.count_launches(1 + 2 + 5 + 7 * 4 + 5 + 2 + 8 + 2 + 1 + 3 * 6)
+    ws = _lib.workspace("cv_head", nbytes, dev, torch.uint8)
+    x = _lib.f32(imgs)
+    _lib.call("nr_cost_volume_head_fwd", sn, _lib.ptr(packed), _lib.ptr(x), _lib.ptr(prob), _lib.ptr(depth_norm), rfn, h, w, _lib.ptr(out),
+              out.shape[-1], out_off, int(encoders.PRECISION == "tf32"), ws.data_ptr(), nbytes, on=imgs,
+              kernels=1 + 2 + 5 + 7 * 4 + 5 + 2 + 8 + 2 + 1 + 3 * 6)
     return out
 
 
@@ -318,14 +274,19 @@ def cost_volume_forward_or_reference(reference_forward):
 SRC_KEY = "_nr_src_imgs_info"      # ref_imgs_info: the source views of the frame being encoded (CostVolumeInitNet), set by the frame renderer
 
 
+def is_cost_volume(module):
+    """True for a CostVolumeInitNet, this package's or the reference's (which carries an `mvsnet`); else a DepthInitNet."""
+    return isinstance(module, CostVolumeInitNet) or hasattr(module, "mvsnet")
+
+
 def init_usable(module, ref_imgs_info):
-    if isinstance(module, CostVolumeInitNet) or hasattr(module, "mvsnet"):
+    if is_cost_volume(module):
         return cost_volume_usable(module, ref_imgs_info, ref_imgs_info.get(SRC_KEY))
     return usable(module, ref_imgs_info)
 
 
 def init_forward_into(module, ref_imgs_info, out, out_off, is_train=False):
     """The owner's init net (DepthInitNet or CostVolumeInitNet) into a slot of the frame pack."""
-    if isinstance(module, CostVolumeInitNet) or hasattr(module, "mvsnet"):
+    if is_cost_volume(module):
         return cost_volume_forward_into(module, ref_imgs_info, ref_imgs_info[SRC_KEY], is_train, out, out_off)
     return forward_into(module, ref_imgs_info, out, out_off)

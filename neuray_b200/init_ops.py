@@ -20,12 +20,9 @@ def get_diff_feats(ref_imgs_info, depth_in):
     rfn, _, h, w = imgs.shape
     if depth_in.shape != (rfn, 1, h, w):
         raise _lib.NeurayB200Error(f"depth_in {tuple(depth_in.shape)} must be [rfn,1,h,w] = {(rfn, 1, h, w)}")
-    f = lambda t: t.detach().float().contiguous()
-    imgs_c, depth_c, poses_c, ks_c = f(imgs), f(depth_in), f(ref_imgs_info["poses"]), f(ref_imgs_info["Ks"])
+    imgs_c, depth_c, poses_c, ks_c = (_lib.f32(t) for t in (imgs, depth_in, ref_imgs_info["poses"], ref_imgs_info["Ks"]))
     _, vp = camera_blocks(None, ref_imgs_info)
     out = torch.empty(rfn, 8, h, w, dtype=torch.float32, device=imgs.device)
-    with _lib.on_device(imgs):
-        _lib.check(_lib.lib().nr_diff_feats(_lib.ptr(imgs_c), _lib.ptr(depth_c), _lib.ptr(poses_c), _lib.ptr(ks_c), _lib.ptr(vp), rfn, h, w,
-                                            _lib.ptr(out), _lib.stream_of(imgs)), "nr_diff_feats")
-    _lib.count_launches(1)
+    _lib.call("nr_diff_feats", _lib.ptr(imgs_c), _lib.ptr(depth_c), _lib.ptr(poses_c), _lib.ptr(ks_c), _lib.ptr(vp), rfn, h, w, _lib.ptr(out),
+              on=imgs)
     return out

@@ -16,10 +16,6 @@ from . import _lib
 from .backward import unpack_point_grads
 
 
-def _f(t):
-    return t.detach().contiguous().float()
-
-
 class _DepthMeanFn(torch.autograd.Function):
     """nr_depth_mean: ray_feats [rfn,32,fh,fw] + coords -> decoder means [rfn,pn,2] of the coarse (and fine) mean head."""
 
@@ -29,15 +25,13 @@ class _DepthMeanFn(torch.autograd.Function):
         rfn, _, fh, fw = ray_feats.shape
         pn = meta["coords"].shape[1]
         dev = ray_feats.device
-        feats = _f(ray_feats)
+        feats = _lib.f32(ray_feats)
         outs = [torch.empty(rfn, pn, 2, dtype=torch.float32, device=dev) for _ in meta["w_point"]]
         p.map, p.coords = _lib.ptr(feats), _lib.ptr(meta["coords"])
         p.rfn, p.pn, p.h, p.w, p.fh, p.fw = rfn, pn, meta["h"], meta["w"], fh, fw
         for k, (wp, o) in enumerate(zip(meta["w_point"], outs)):
             p.w_point[k], p.mean[k] = _lib.ptr(wp), _lib.ptr(o)
-        with _lib.on_device(ray_feats):
-            _lib.check(_lib.lib().nr_depth_mean(C.byref(p), _lib.stream_of(ray_feats)), "nr_depth_mean")
-        _lib.count_launches(1)
+        _lib.call("nr_depth_mean", C.byref(p), on=ray_feats)
         ctx.meta, ctx.feats = meta, feats
         ctx.need_feats = ray_feats.requires_grad
         ctx.need = [t.requires_grad for t in params]
@@ -54,15 +48,13 @@ class _DepthMeanFn(torch.autograd.Function):
         d_map = torch.zeros_like(feats) if ctx.need_feats else None
         keep, d_w = [], []
         for k, wp in enumerate(meta["w_point"]):
-            gk = _f(g[k]) if g[k] is not None else torch.zeros(rfn, p.pn, 2, dtype=torch.float32, device=dev)
+            gk = _lib.f32(g[k]) if g[k] is not None else torch.zeros(rfn, p.pn, 2, dtype=torch.float32, device=dev)
             dw = torch.zeros(wp.numel(), dtype=torch.float32, device=dev)
             keep.append(gk)
             d_w.append(dw)
             p.w_point[k], p.d_mean[k], p.d_w_point[k] = _lib.ptr(wp), _lib.ptr(gk), _lib.ptr(dw)
         p.d_map = _lib.ptr(d_map)
-        with _lib.on_device(feats):
-            _lib.check(_lib.lib().nr_depth_mean(C.byref(p), _lib.stream_of(feats)), "nr_depth_mean (backward)")
-        _lib.count_launches(1)
+        _lib.call("nr_depth_mean", C.byref(p), on=feats, what="nr_depth_mean (backward)")
         grads = {}
         for k, (names, imap) in enumerate(zip(meta["names"], meta["index_maps"])):
             got = unpack_point_grads(imap, d_w[k])
@@ -81,7 +73,7 @@ def gen_depth_loss_coords(h, w, num, device):
 def predict_mean_for_depth_loss(self, ref_imgs_info):
     """NeuralRayGenRenderer.predict_mean_for_depth_loss (renderer.py:280-316) for an owner with dist_decoder
     (/ fine_dist_decoder) under the reference's parameter names; returns the same dict."""
-    from .renderer import pass_index_map, pass_weights
+    from .renderer import pass_index_map, pass_params, pass_weights
     ray_feats, ref_imgs = ref_imgs_info["ray_feats"], ref_imgs_info["imgs"]
     if not ray_feats.is_cuda:
         raise _lib.NeurayB200Error("predict_mean_for_depth_loss needs CUDA tensors (no CPU fallback)")
@@ -89,14 +81,14 @@ def predict_mean_for_depth_loss(self, ref_imgs_info):
     coords = gen_depth_loss_coords(h, w, self.cfg["depth_loss_coords_num"], ref_imgs.device)
     coords = coords.unsqueeze(0).repeat(rfn, 1, 1)
     fine = bool(self.cfg["use_hierarchical_sampling"])
-    decs = [("dist_decoder", self.dist_decoder, False)] + ([("fine_dist_decoder", self.fine_dist_decoder, True)] if fine else [])
     w_point, names, index_maps, params, param_names = [], [], [], [], []
-    for dec_name, dec, is_fine in decs:
+    for is_fine in (False, True) if fine else (False,):
         dn = self.cfg["fine_depth_sample_num" if is_fine else "depth_sample_num"]
         if is_fine and self.cfg["fine_depth_use_all"]:
             dn += self.cfg["depth_sample_num"]
         w_point.append(pass_weights(self, is_fine, dn, ray_feats.device)[0])
-        own = {f"{dec_name}.{k}": v for k, v in dec.named_parameters() if k.startswith("mean_decoder.")}
+        _, _, dec_name, _, allp = pass_params(self, is_fine)
+        own = {n: v for n, v in allp.items() if n.startswith(f"{dec_name}.mean_decoder.")}
         index_maps.append(pass_index_map(self, is_fine, ray_feats.device))     # covers the whole pass; only the mean head gets a gradient here
         names.append(list(own))
         params += list(own.values())
@@ -115,13 +107,10 @@ class _RenderLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, pr, gt, mask):
         qn, rn, _ = pr.shape
-        a, b = _f(pr), _f(gt)
+        a, b = _lib.f32(pr), _lib.f32(gt)
         m = None if mask is None else mask.detach().contiguous().to(torch.uint8)
         loss = torch.empty(qn, dtype=torch.float32, device=pr.device)
-        with _lib.on_device(pr):
-            _lib.check(_lib.lib().nr_render_loss(_lib.ptr(a), _lib.ptr(b), _lib.ptr(m), qn, rn, _lib.ptr(loss), None, None, _lib.stream_of(pr)),
-                       "nr_render_loss")
-        _lib.count_launches(1)
+        _lib.call("nr_render_loss", _lib.ptr(a), _lib.ptr(b), _lib.ptr(m), qn, rn, _lib.ptr(loss), None, None, on=pr)
         ctx.keep = (a, b, m)
         return loss
 
@@ -130,11 +119,9 @@ class _RenderLossFn(torch.autograd.Function):
         a, b, m = ctx.keep
         qn, rn, _ = a.shape
         d = torch.empty_like(a)
-        gg = _f(g)
-        with _lib.on_device(a):
-            _lib.check(_lib.lib().nr_render_loss(_lib.ptr(a), _lib.ptr(b), _lib.ptr(m), qn, rn, None, _lib.ptr(gg), _lib.ptr(d), _lib.stream_of(a)),
-                       "nr_render_loss (backward)")
-        _lib.count_launches(1)
+        gg = _lib.f32(g)
+        _lib.call("nr_render_loss", _lib.ptr(a), _lib.ptr(b), _lib.ptr(m), qn, rn, None, _lib.ptr(gg), _lib.ptr(d), on=a,
+                  what="nr_render_loss (backward)")
         return d, (-d if ctx.needs_input_grad[1] else None), None
 
 
@@ -151,13 +138,11 @@ class _DepthLossFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, meta, depth_pr):
-        x = _f(depth_pr)
+        x = _lib.f32(depth_pr)
         loss = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         p = _DepthLossFn._params(meta, x)
         p.loss = _lib.ptr(loss)
-        with _lib.on_device(x):
-            _lib.check(_lib.lib().nr_depth_loss(C.byref(p), _lib.stream_of(x)), "nr_depth_loss")
-        _lib.count_launches(1)
+        _lib.call("nr_depth_loss", C.byref(p), on=x)
         ctx.meta, ctx.x = meta, x
         return loss
 
@@ -165,25 +150,20 @@ class _DepthLossFn(torch.autograd.Function):
     def backward(ctx, g):
         x = ctx.x
         d = torch.empty_like(x)
-        gg = _f(g)
+        gg = _lib.f32(g)
         p = _DepthLossFn._params(ctx.meta, x)
         p.g, p.d_depth_pr = _lib.ptr(gg), _lib.ptr(d)
-        with _lib.on_device(x):
-            _lib.check(_lib.lib().nr_depth_loss(C.byref(p), _lib.stream_of(x)), "nr_depth_loss (backward)")
-        _lib.count_launches(1)
+        _lib.call("nr_depth_loss", C.byref(p), on=x, what="nr_depth_loss (backward)")
         return None, d
 
 
 class _ConsistencyFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, prob0, prob1):
-        a, b = _f(prob0), _f(prob1)
+        a, b = _lib.f32(prob0), _lib.f32(prob1)
         qn, rn, dn = b.shape
         loss = torch.empty(qn, dtype=torch.float32, device=b.device)
-        with _lib.on_device(b):
-            _lib.check(_lib.lib().nr_consistency_loss(_lib.ptr(a), _lib.ptr(b), qn, rn, dn, _lib.ptr(loss), None, None, _lib.stream_of(b)),
-                       "nr_consistency_loss")
-        _lib.count_launches(1)
+        _lib.call("nr_consistency_loss", _lib.ptr(a), _lib.ptr(b), qn, rn, dn, _lib.ptr(loss), None, None, on=b)
         ctx.keep = (a, b)
         return loss
 
@@ -192,11 +172,9 @@ class _ConsistencyFn(torch.autograd.Function):
         a, b = ctx.keep
         qn, rn, dn = b.shape
         d = torch.empty_like(b)
-        gg = _f(g)
-        with _lib.on_device(b):
-            _lib.check(_lib.lib().nr_consistency_loss(_lib.ptr(a), _lib.ptr(b), qn, rn, dn, None, _lib.ptr(gg), _lib.ptr(d), _lib.stream_of(b)),
-                       "nr_consistency_loss (backward)")
-        _lib.count_launches(1)
+        gg = _lib.f32(g)
+        _lib.call("nr_consistency_loss", _lib.ptr(a), _lib.ptr(b), qn, rn, dn, None, _lib.ptr(gg), _lib.ptr(d), on=b,
+                  what="nr_consistency_loss (backward)")
         return None, d
 
 
@@ -263,8 +241,8 @@ class DepthLoss(Loss):
         depth_maps = ref["true_depth"]
         rfn, _, h, w = depth_maps.shape
         gso = data_gt["scene_name"].startswith("gso")
-        meta = {"coords": _f(data_pr["depth_coords"]), "true_depth": _f(depth_maps), "aug_depth": _f(ref["depth"]) if gso else None,
-                "depth_range": _f(ref["depth_range"]), "h": h, "w": w, "loss_type": 0 if self.cfg["depth_loss_type"] == "l2" else 1,
+        meta = {"coords": _lib.f32(data_pr["depth_coords"]), "true_depth": _lib.f32(depth_maps), "aug_depth": _lib.f32(ref["depth"]) if gso else None,
+                "depth_range": _lib.f32(ref["depth_range"]), "h": h, "w": w, "loss_type": 0 if self.cfg["depth_loss_type"] == "l2" else 1,
                 "beta": float(self.cfg["depth_loss_l1_beta"]), "thresh": float(self.cfg["depth_correct_thresh"])}
         outputs = {"loss_depth": _DepthLossFn.apply(meta, data_pr["depth_mean"])}
         if "depth_mean_fine" in data_pr:

@@ -26,15 +26,6 @@ __all__ = [
 ]
 
 
-def _c(t):
-    return t.contiguous().float()
-
-
-def _ck(rc, what):
-    _lib.check(rc, what)
-    _lib.count_launches(1)
-
-
 def _no_grad_inputs(what, **tensors):
     """These launchers have no backward: refuse inputs that would need one (see the module docstring)."""
     if torch.is_grad_enabled():
@@ -53,55 +44,49 @@ def coords2rays(coords, poses, Ks):
     """reference render_ops.py:4-25.  coords [n,rn,2], poses [n,3,4], Ks [n,3,3] -> centers, directions [n,rn,3]."""
     _no_grad_inputs("coords2rays", coords=coords, poses=poses, Ks=Ks)
     n, rn, _ = coords.shape
-    coords = _c(coords)
+    coords = _lib.f32(coords)
     centers = torch.empty(n, rn, 3, dtype=torch.float32, device=coords.device)
     dirs = torch.empty_like(centers)
-    with _lib.on_device(coords):
-        for i in range(n):
-            cam = _cam_of(poses, Ks, i)
-            _ck(_lib.lib().nr_coords2rays(_lib.ptr(coords[i]), _lib.ptr(cam), rn, _lib.ptr(centers[i]), _lib.ptr(dirs[i]),
-                                          _lib.stream_of(coords)), "nr_coords2rays")
+    for i in range(n):
+        cam = _cam_of(poses, Ks, i)
+        _lib.call("nr_coords2rays", _lib.ptr(coords[i]), _lib.ptr(cam), rn, _lib.ptr(centers[i]), _lib.ptr(dirs[i]), on=coords)
     return centers, dirs
 
 
 def depth2points(que_imgs_info, que_depth):
     """reference render_ops.py:27-39 -> que_pts, que_dir [qn,rn,dn,3]."""
     _no_grad_inputs("depth2points", coords=que_imgs_info["coords"], que_depth=que_depth, poses=que_imgs_info["poses"])
-    coords = _c(que_imgs_info["coords"])
-    que_depth = _c(que_depth)
+    coords = _lib.f32(que_imgs_info["coords"])
+    que_depth = _lib.f32(que_depth)
     qn, rn, dn = que_depth.shape
     pts = torch.empty(qn, rn, dn, 3, dtype=torch.float32, device=coords.device)
     dirs = torch.empty_like(pts)
-    with _lib.on_device(coords):
-        for i in range(qn):
-            cam = _cam_of(que_imgs_info["poses"], que_imgs_info["Ks"], i)
-            _ck(_lib.lib().nr_depth2points(_lib.ptr(coords[i]), _lib.ptr(cam), _lib.ptr(que_depth[i]), rn, dn,
-                                           _lib.ptr(pts[i]), _lib.ptr(dirs[i]), _lib.stream_of(coords)), "nr_depth2points")
+    for i in range(qn):
+        cam = _cam_of(que_imgs_info["poses"], que_imgs_info["Ks"], i)
+        _lib.call("nr_depth2points", _lib.ptr(coords[i]), _lib.ptr(cam), _lib.ptr(que_depth[i]), rn, dn, _lib.ptr(pts[i]), _lib.ptr(dirs[i]),
+                  on=coords)
     return pts, dirs
 
 
 def depth2dists(depth):
     """reference render_ops.py:41-44."""
     _no_grad_inputs("depth2dists", depth=depth)
-    depth = _c(depth)
+    depth = _lib.f32(depth)
     out = torch.empty_like(depth)
     dn = depth.shape[-1]
-    with _lib.on_device(depth):
-        _ck(_lib.lib().nr_depth2dists(_lib.ptr(depth), depth.numel() // dn, dn, _lib.ptr(out), _lib.stream_of(depth)), "nr_depth2dists")
+    _lib.call("nr_depth2dists", _lib.ptr(depth), depth.numel() // dn, dn, _lib.ptr(out), on=depth)
     return out
 
 
 def depth2inv_dists(depth, depth_range):
     """reference render_ops.py:46-52.  depth [qn,rn,dn], depth_range [qn,2]."""
     _no_grad_inputs("depth2inv_dists", depth=depth)
-    depth = _c(depth)
+    depth = _lib.f32(depth)
     out = torch.empty_like(depth)
     qn, rn, dn = depth.shape
-    dr = _c(depth_range.detach())
-    with _lib.on_device(depth):
-        for i in range(qn):
-            _ck(_lib.lib().nr_depth2inv_dists(_lib.ptr(depth[i]), _lib.ptr(dr[i]), rn, dn, _lib.ptr(out[i]), _lib.stream_of(depth)),
-                "nr_depth2inv_dists")
+    dr = _lib.f32(depth_range)
+    for i in range(qn):
+        _lib.call("nr_depth2inv_dists", _lib.ptr(depth[i]), _lib.ptr(dr[i]), rn, dn, _lib.ptr(out[i]), on=depth)
     return out
 
 
@@ -110,14 +95,13 @@ class _InterpFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, feats, points, mask, h, w, border, align):
-        f, pts = _c(feats.detach()), _c(points.detach())
-        m = _c(mask.detach()) if mask is not None else None
+        f, pts = _lib.f32(feats), _lib.f32(points)
+        m = _lib.f32(mask) if mask is not None else None
         b, c, ch, cw = f.shape
         n = pts.shape[1]
         out = torch.empty(b, n, c, dtype=torch.float32, device=f.device)
-        with _lib.on_device(f):
-            _ck(_lib.lib().nr_interpolate_feats(_lib.ptr(f), _lib.ptr(pts), _lib.ptr(m), b, c, ch, cw, n, float(h), float(w), border, align,
-                                                _lib.ptr(out), _lib.stream_of(f)), "nr_interpolate_feats")
+        _lib.call("nr_interpolate_feats", _lib.ptr(f), _lib.ptr(pts), _lib.ptr(m), b, c, ch, cw, n, float(h), float(w), border, align,
+                  _lib.ptr(out), on=f)
         ctx.save_for_backward(pts, m)
         ctx.geom = (b, c, ch, cw, n, float(h), float(w), border, align)
         return out
@@ -126,11 +110,9 @@ class _InterpFn(torch.autograd.Function):
     def backward(ctx, g):
         pts, m = ctx.saved_tensors
         b, c, ch, cw, n, h, w, border, align = ctx.geom
-        g = _c(g)
+        g = _lib.f32(g)
         d_feats = torch.zeros(b, c, ch, cw, dtype=torch.float32, device=g.device)
-        with _lib.on_device(g):
-            _ck(_lib.lib().nr_interpolate_feats_bwd(_lib.ptr(g), _lib.ptr(pts), _lib.ptr(m), b, c, ch, cw, n, h, w, border, align,
-                                                    _lib.ptr(d_feats), _lib.stream_of(g)), "nr_interpolate_feats_bwd")
+        _lib.call("nr_interpolate_feats_bwd", _lib.ptr(g), _lib.ptr(pts), _lib.ptr(m), b, c, ch, cw, n, h, w, border, align, _lib.ptr(d_feats), on=g)
         return d_feats, None, None, None, None, None, None
 
 
@@ -160,18 +142,16 @@ def interpolate_feature_map(ray_feats, coords, mask, h, w, border_type="border")
 def alpha_values2hit_prob(alpha_values):
     """reference render_ops.py:72-80."""
     _no_grad_inputs("alpha_values2hit_prob", alpha_values=alpha_values)
-    a = _c(alpha_values)
+    a = _lib.f32(alpha_values)
     out = torch.empty_like(a)
     dn = a.shape[-1]
-    with _lib.on_device(a):
-        _ck(_lib.lib().nr_alpha_values2hit_prob(_lib.ptr(a), a.numel() // dn, dn, _lib.ptr(out), _lib.stream_of(a)),
-            "nr_alpha_values2hit_prob")
+    _lib.call("nr_alpha_values2hit_prob", _lib.ptr(a), a.numel() // dn, dn, _lib.ptr(out), on=a)
     return out
 
 
 def _project(pts, poses, Ks, h, w, want_dir):
     _no_grad_inputs("project_points", pts=pts, poses=poses, Ks=Ks)
-    pts = _c(pts)
+    pts = _lib.f32(pts)
     pn = pts.shape[0]
     rfn = poses.shape[0]
     _, vp = camera_blocks(None, {"poses": poses, "Ks": Ks})
@@ -181,9 +161,8 @@ def _project(pts, poses, Ks, h, w, want_dir):
     mask = torch.empty(rfn, pn, dtype=torch.float32, device=dev)
     valid = torch.empty(rfn, pn, dtype=torch.float32, device=dev)
     d = torch.empty(rfn, pn, 3, dtype=torch.float32, device=dev) if want_dir else None
-    with _lib.on_device(pts):
-        _ck(_lib.lib().nr_project_points(_lib.ptr(pts), pn, _lib.ptr(vp), rfn, int(h), int(w), _lib.ptr(d), _lib.ptr(pix),
-                                         _lib.ptr(depth), _lib.ptr(mask), _lib.ptr(valid), _lib.stream_of(pts)), "nr_project_points")
+    _lib.call("nr_project_points", _lib.ptr(pts), pn, _lib.ptr(vp), rfn, int(h), int(w), _lib.ptr(d), _lib.ptr(pix), _lib.ptr(depth),
+              _lib.ptr(mask), _lib.ptr(valid), on=pts)
     return d, pix, depth, mask, valid
 
 
@@ -227,13 +206,12 @@ def sample_depth(depth_range, coords, sample_num, random_sample):
     dev = coords.device
     depth = torch.empty(qn, rn, dn, dtype=torch.float32, device=dev)
     dists = torch.empty_like(depth)
-    dr = _c(depth_range.detach())
+    dr = _lib.f32(depth_range)
     # the uniforms come from torch's generator exactly like the reference's torch.rand(..., device=device)
     jitter = torch.rand(qn, rn, dn - 2, dtype=torch.float32, device=dev) if random_sample else None
-    with _lib.on_device(coords):
-        for i in range(qn):
-            _ck(_lib.lib().nr_sample_depth(_lib.ptr(dr[i]), rn, dn, _lib.ptr(jitter[i]) if jitter is not None else None,
-                                           _lib.ptr(depth[i]), _lib.ptr(dists[i]), _lib.stream_of(coords)), "nr_sample_depth")
+    for i in range(qn):
+        _lib.call("nr_sample_depth", _lib.ptr(dr[i]), rn, dn, _lib.ptr(jitter[i]) if jitter is not None else None, _lib.ptr(depth[i]),
+                  _lib.ptr(dists[i]), on=coords)
     return depth, dists
 
 
@@ -246,22 +224,21 @@ def fine_sample_u(fdn, device):
 def sample_fine_depth(depth, hit_prob, depth_range, sample_num, random_sample, inv_mode=True):
     """reference render_ops.py:172-229 -> [qn,rn,sample_num] (unsorted)."""
     _no_grad_inputs("sample_fine_depth", depth=depth, hit_prob=hit_prob)
-    depth, hit_prob = _c(depth), _c(hit_prob)
+    depth, hit_prob = _lib.f32(depth), _lib.f32(hit_prob)
     qn, rn, dn = depth.shape
     fdn = int(sample_num)
     dev = depth.device
     out = torch.empty(qn, rn, fdn, dtype=torch.float32, device=dev)
     # the reference uses depth_range[0] for every query (render_ops.py:183)
-    dr = _c(depth_range.detach()[0]) if inv_mode else None
+    dr = _lib.f32(depth_range[0]) if inv_mode else None
     if random_sample:
         u = torch.rand([qn, rn, fdn]).to(dev).contiguous()      # CPU generator, like render_ops.py:205
         stride = fdn
     else:
         u = fine_sample_u(fdn, dev)
         stride = 0
-    with _lib.on_device(depth):
-        for i in range(qn):
-            ui = u[i] if random_sample else u
-            _ck(_lib.lib().nr_sample_fine_depth(_lib.ptr(depth[i]), _lib.ptr(hit_prob[i]), _lib.ptr(dr), rn, dn, fdn, _lib.ptr(ui), stride,
-                                                0, 0, _lib.ptr(out[i]), _lib.stream_of(depth)), "nr_sample_fine_depth")
+    for i in range(qn):
+        ui = u[i] if random_sample else u
+        _lib.call("nr_sample_fine_depth", _lib.ptr(depth[i]), _lib.ptr(hit_prob[i]), _lib.ptr(dr), rn, dn, fdn, _lib.ptr(ui), stride, 0, 0,
+                  _lib.ptr(out[i]), on=depth)
     return out

@@ -23,7 +23,7 @@ import torch.nn as nn
 
 from . import _lib, encoders, init_nets, modules
 from .render_ops import fine_sample_u, interpolate_feats, sample_depth
-from .weights import camera_blocks, pack_pass, point_index_map, posenc_table
+from .weights import camera_blocks, pack_pass, point_index_map, posenc_table, stamp
 
 PACK_KEY = "_nr_frame_pack"        # ref_imgs_info: the FramePack of the frame being rendered (lives for one render() call)
 CAM_KEY = "_nr_que_cam"            # que_imgs_info: que_cam block of the frame being rendered (same lifetime)
@@ -41,24 +41,6 @@ base_cfg = {
     # NeuralRayGenRenderer.default_cfg (renderer.py:256-261), read by predict_mean_for_depth_loss
     "use_depth_loss": False, "depth_loss_coords_num": 8192,
 }
-
-
-# Grow-only device workspaces, reused across passes, chunks and frames.  The C-ABI never allocates (the caller owns
-# the workspace); taking 335 MB of point records per pass and 246 MB of repacked maps per frame from torch's caching
-# allocator every time fragmented it (small long-lived outputs land in the freed big blocks) and cost cudaMalloc calls
-# in steady state (tools/e2e_breakdown.py).  Everything is stream-ordered on the caller's current stream; rendering
-# with one network object from several streams at once is not supported.
-_WORKSPACES = {}
-
-
-def _workspace(key, numel, dev):
-    buf = _WORKSPACES.get((key, str(dev)))
-    if buf is None or buf.numel() < numel:
-        buf = None
-        _WORKSPACES.pop((key, str(dev)), None)
-        buf = torch.empty(numel, dtype=torch.float32, device=dev)
-        _WORKSPACES[(key, str(dev))] = buf
-    return buf[:numel]
 
 
 _PACK_POOL = {}      # (device, feat shape, rgb shape) -> [(feat, rgb)] of dropped FramePacks, at most two kept
@@ -94,7 +76,7 @@ class FramePack:
         if encoder_owner is not None:
             fh, fw = encoders.image_dims(h, w)
             if rf is None:       # the owner's init net writes its ray_feats straight into the pack (encoders.encode_frame)
-                if not hasattr(encoder_owner.init_net, "mvsnet") and init_nets.dims(h, w) != (fh, fw):
+                if not init_nets.is_cost_volume(encoder_owner.init_net) and init_nets.dims(h, w) != (fh, fw):
                     raise _lib.NeurayB200Error(f"init net and image encoder disagree on the map size for {h}x{w} images")
             elif tuple(rf.shape[-2:]) != (fh, fw) or rf.shape[1] != 32:
                 raise _lib.NeurayB200Error(f"ray_feats {tuple(rf.shape)} do not match the image encoder's output size {(fh, fw)} for {h}x{w} images")
@@ -117,19 +99,14 @@ class FramePack:
         else:
             self.feat = torch.empty(rfn, fh, fw, 64, dtype=torch.float32, device=dev)
             self.rgb = torch.empty(rfn, h, w, 4, dtype=torch.float32, device=dev)
-        if encoder_owner is not None:
+        if encoder_owner is not None:      # the encoders write the feature maps; only the images are repacked below
             encoders.encode_frame(encoder_owner, ref_imgs_info, self.feat)
-            with _lib.on_device(imgs):
-                _lib.check(_lib.lib().nr_pack_feature_maps(None, None, _lib.ptr(imgs.detach().contiguous().float()), rfn, h, w, fh, fw,
-                                                           None, _lib.ptr(self.rgb), _lib.stream_of(imgs)), "nr_pack_feature_maps (rgb)")
-            _lib.count_launches(1)
+            rf_c = imf_c = feat = None
         else:
-            with _lib.on_device(imgs):
-                _lib.check(_lib.lib().nr_pack_feature_maps(
-                    _lib.ptr(rf.detach().contiguous().float()), _lib.ptr(imf.detach().contiguous().float()),
-                    _lib.ptr(imgs.detach().contiguous().float()), rfn, h, w, fh, fw, _lib.ptr(self.feat), _lib.ptr(self.rgb),
-                    _lib.stream_of(imgs)), "nr_pack_feature_maps")
-            _lib.count_launches(2)
+            rf_c, imf_c, feat = _lib.f32(rf), _lib.f32(imf), self.feat
+        imgs_c = _lib.f32(imgs)
+        _lib.call("nr_pack_feature_maps", _lib.ptr(rf_c), _lib.ptr(imf_c), _lib.ptr(imgs_c), rfn, h, w, fh, fw, _lib.ptr(feat), _lib.ptr(self.rgb),
+                  on=imgs, kernels=1 if feat is None else 2)
         _, self.view_params = camera_blocks(None, ref_imgs_info)
         self.src = tuple((ref_imgs_info[k], ref_imgs_info[k]._version) for k in _PACK_SOURCES)
 
@@ -146,27 +123,29 @@ def frame_pack(ref_imgs_info):
     return pack
 
 
-def _pass_modules(owner, is_fine):
-    return (owner.fine_dist_decoder, owner.fine_agg_net, "fine_dist_decoder", "fine_agg_net") if is_fine else \
+def pass_params(owner, is_fine):
+    """(dec, agg, dec_name, agg_name, {state-dict name: parameter}) of the coarse or the fine pass, decoder parameters first."""
+    dec, agg, dec_name, agg_name = (owner.fine_dist_decoder, owner.fine_agg_net, "fine_dist_decoder", "fine_agg_net") if is_fine else \
         (owner.dist_decoder, owner.agg_net, "dist_decoder", "agg_net")
+    params = {f"{dec_name}.{k}": v for k, v in dec.named_parameters()}
+    params.update({f"{agg_name}.{k}": v for k, v in agg.named_parameters()})
+    return dec, agg, dec_name, agg_name, params
 
 
 def pass_weights(owner, is_fine, dn, device):
     """Packed weights of one pass (nr_pack_weights), cached on the owner and re-packed when any parameter changed
     (optimizer steps bump tensor._version).  Every re-pack gets fresh buffers: an autograd graph recorded before the
     parameter update keeps reading the buffers it was recorded with."""
-    dec, agg, dec_name, agg_name = _pass_modules(owner, is_fine)
-    params = {f"{dec_name}.{k}": v for k, v in dec.named_parameters()}
-    params.update({f"{agg_name}.{k}": v for k, v in agg.named_parameters()})
-    stamp = tuple((v.data_ptr(), v._version) for v in params.values()) + (str(device),)
+    _, agg, dec_name, agg_name, params = pass_params(owner, is_fine)
+    st = stamp(params.values(), str(device))
     cache = owner.__dict__.setdefault("_nr_wcache", {})
     hit = cache.get(is_fine)
-    if hit is None or hit[0] != stamp:
+    if hit is None or hit[0] != st:
         first = next(iter(params.values()))
         if first.device != torch.device(device):
             raise _lib.NeurayB200Error(f"parameters live on {first.device} but the rays are on {device}")
         wp, wr, wt = pack_pass(params, dec_name, agg_name)
-        hit = (stamp, wp, wr, hit[3] if hit is not None else {}, wt)
+        hit = (st, wp, wr, hit[3] if hit is not None else {}, wt)
         cache[is_fine] = hit
     pe = hit[3].get(dn)
     if pe is None:
@@ -182,9 +161,7 @@ def pass_weights(owner, is_fine, dn, device):
 
 def pass_index_map(owner, is_fine, dev):
     """weights.point_index_map of a pass (packed w_point position -> parameter element), cached on the owner."""
-    dec, agg, dec_name, agg_name = _pass_modules(owner, is_fine)
-    allp = {f"{dec_name}.{k}": v for k, v in dec.named_parameters()}
-    allp.update({f"{agg_name}.{k}": v for k, v in agg.named_parameters()})
+    _, _, dec_name, agg_name, allp = pass_params(owner, is_fine)
     maps = owner.__dict__.setdefault("_nr_index_maps", {})
     key = (is_fine, str(dev), tuple(allp))
     if key not in maps:
@@ -198,19 +175,18 @@ def _check_supported(owner):
         raise NotImplementedError("use_dr_prediction (direct rendering / SH fit) is outside the B200 hot path (SURVEY.md 8f)")
 
 
-def _launch_pass(owner, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine, want_hit):
-    """Enqueues the two kernels of one pass; returns the raw output dict (ray_mask as uint8)."""
+def _launch_pass(owner, dec, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine, want_hit):
+    """Enqueues the two kernels of one pass (dec: its distance decoder); returns the raw output dict (ray_mask as uint8)."""
     cfg = owner.cfg
     coords = que_imgs_info["coords"]
     dev = coords.device
     pack = frame_pack(ref_imgs_info)
     _, rn, dn = que_depth.shape
-    dec, agg, _, _ = _pass_modules(owner, is_fine)
     w_point, w_ray, pos_enc, w_tc = pass_weights(owner, is_fine, dn, dev)
     cam = que_imgs_info.get(CAM_KEY)
     if cam is None:
         cam, _ = camera_blocks(que_imgs_info, None)
-    coords_c = coords[0].detach().contiguous().float()
+    coords_c = _lib.f32(coords[0])
 
     out = {
         "pixel_colors": torch.empty(1, rn, 3, dtype=torch.float32, device=dev),
@@ -218,7 +194,7 @@ def _launch_pass(owner, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine, 
         "render_depth": torch.empty(1, rn, dtype=torch.float32, device=dev),
         "ray_mask_u8": torch.empty(1, rn, dtype=torch.uint8, device=dev),
     }
-    rec = _workspace("point_rec", rn * dn * _lib.NR_POINT_REC, dev)
+    rec = _lib.workspace("point_rec", rn * dn * _lib.NR_POINT_REC, dev, torch.float32)
     p = _lib.NrPassParams()
     p.coords, p.que_depth, p.que_cam = _lib.ptr(coords_c), _lib.ptr(que_depth), _lib.ptr(cam)
     p.rn, p.dn = rn, dn
@@ -244,19 +220,18 @@ def _launch_pass(owner, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine, 
     if rn == 0:          # nothing to render: the (empty) outputs are already in place
         out["_bwd"] = None
         return out
-    with _lib.on_device(coords):
-        if _lib.PROFILE is not None:
-            # bench.py: time the dominant kernel alone, with CUDA events on the launching stream
+    if _lib.PROFILE is not None:
+        # bench.py: time the dominant kernel alone, with CUDA events on the launching stream
+        with _lib.on_device(coords):      # Event.record() records on the current device's stream
             e0, e1, e2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
             e0.record()
-            _lib.check(_lib.lib().nr_point_kernel(C.byref(p), stream), "nr_point_kernel")
+            _lib.call("nr_point_kernel", C.byref(p), on=coords)
             e1.record()
-            _lib.check(_lib.lib().nr_ray_kernel(C.byref(p), stream), "nr_ray_kernel")
+            _lib.call("nr_ray_kernel", C.byref(p), on=coords)
             e2.record()
-            _lib.PROFILE.append((e0, e1, rn * dn, e2))
-        else:
-            _lib.check(_lib.lib().nr_render_pass_fwd(C.byref(p), stream), "nr_render_pass_fwd")
-    _lib.count_launches(2)
+        _lib.PROFILE.append((e0, e1, rn * dn, e2))
+    else:
+        _lib.call("nr_render_pass_fwd", C.byref(p), on=coords, kernels=2)
     # what nr_render_pass_bwd needs to run on the same inputs (kept alive by the autograd node, dropped otherwise)
     out["_bwd"] = (p, (coords_c, que_depth, cam, pack, w_point, w_ray, pos_enc, w_tc), (pack.rfn, pack.fh, pack.fw, 64), stream)
     return out
@@ -273,22 +248,21 @@ def run_pass(owner, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine=None,
     coords = que_imgs_info["coords"]
     if coords.shape[0] != 1:
         raise _lib.NeurayB200Error("one query view per call (qn == 1), like every call site of the reference")
-    que_depth = que_depth.detach().contiguous().float()
+    que_depth = _lib.f32(que_depth)
     _, rn, dn = que_depth.shape
     if dn > _lib.NR_MAX_SAMPLES:
         raise _lib.NeurayB200Error(f"at most {_lib.NR_MAX_SAMPLES} samples per ray per pass, got {dn}")
-    dec, agg, dec_name, agg_name = _pass_modules(owner, is_fine)
+    dec, _, dec_name, agg_name, params = pass_params(owner, is_fine)
     rf, imf = ref_imgs_info["ray_feats"], ref_imgs_info["img_feats"]
-    named = [(f"{dec_name}.{k}", v) for k, v in dec.named_parameters()] + [(f"{agg_name}.{k}", v) for k, v in agg.named_parameters()]
-    needs_grad = torch.is_grad_enabled() and (rf.requires_grad or imf.requires_grad or any(v.requires_grad for _, v in named))
-    launch = lambda: _launch_pass(owner, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine, want_hit)
+    needs_grad = torch.is_grad_enabled() and (rf.requires_grad or imf.requires_grad or any(v.requires_grad for v in params.values()))
+    launch = lambda: _launch_pass(owner, dec, que_depth, que_imgs_info, ref_imgs_info, is_fine, fine, want_hit)
     if not needs_grad:
         out = launch()
         out.pop("_bwd", None)
     else:
         from .backward import RenderPassFn
-        meta = {"names": [n for n, _ in named], "dec": dec_name, "agg": agg_name}
-        res = RenderPassFn.apply(launch, meta, rf, imf, *[v for _, v in named])
+        meta = {"names": list(params), "dec": dec_name, "agg": agg_name}
+        res = RenderPassFn.apply(launch, meta, rf, imf, *params.values())
         out = {"pixel_colors": res[0], "hit_prob": res[1], "render_depth": res[2], "ray_mask_u8": res[3]}
         if fine:
             out["fine_depth"] = res[4]
@@ -311,7 +285,7 @@ def _finish_outputs(owner, res, que_depth, que_imgs_info):
 def _self_hit_prob(self, que_depth, que_imgs_info, is_fine):
     """a17 predict_self_hit_prob (reference renderer.py:137-155): the query view's own ray_feats decoded along its rays
     (fine-tuning configs).  nr_self_hit_prob, forward and backward."""
-    dec, _, dec_name, _ = _pass_modules(self, is_fine)
+    dec, _, dec_name, _, allp = pass_params(self, is_fine)
     feats = que_imgs_info["ray_feats"]
     coords = que_imgs_info["coords"]
     h, w = que_imgs_info["imgs"].shape[-2:]
@@ -321,11 +295,11 @@ def _self_hit_prob(self, que_depth, que_imgs_info, is_fine):
     dev = coords.device
     _, rn, dn = que_depth.shape
     w_point = pass_weights(self, is_fine, dn, dev)[0]
-    dec_params = {f"{dec_name}.{k}": v for k, v in dec.named_parameters()}
+    dec_params = {n: v for n, v in allp.items() if n.startswith(dec_name + ".")}
     index_map = pass_index_map(self, is_fine, dev)
-    fmap = feats[0].detach().contiguous().float()
-    cc, qd = coords[0].detach().contiguous().float(), que_depth[0].detach().contiguous().float()
-    rng = que_imgs_info["depth_range"][0].detach().float().contiguous()
+    fmap = _lib.f32(feats[0])
+    cc, qd = _lib.f32(coords[0]), _lib.f32(que_depth[0])
+    rng = _lib.f32(que_imgs_info["depth_range"][0])
     use_vis, var_bias = 1 if dec.cfg["use_vis"] else 0, float(dec.cfg["bias_val"])
 
     def params():

@@ -72,12 +72,53 @@ def pack_pass(params, dec, agg, out=None):
         out = (torch.empty(L.total_point, dtype=torch.float32, device=dev), torch.empty(L.total_ray, dtype=torch.float32, device=dev),
                torch.empty(T.total, dtype=torch.float32, device=dev))
     w, keep = pass_weight_struct(params, dec, agg)
-    with _lib.on_device(any_t):
-        _lib.check(_lib.lib().nr_pack_weights(C.byref(w), _lib.ptr(out[0]), _lib.ptr(out[1]), _lib.ptr(out[2]), _lib.stream_of(any_t)),
-                   "nr_pack_weights")
-    _lib.count_launches(1)
+    _lib.call("nr_pack_weights", C.byref(w), _lib.ptr(out[0]), _lib.ptr(out[1]), _lib.ptr(out[2]), on=any_t)
     del keep
     return out
+
+
+def named_tensors(module):
+    """The module's parameters and buffers by state-dict name."""
+    return {**dict(module.named_parameters()), **dict(module.named_buffers())}
+
+
+def has_names(module, names):
+    """True when the module has every one of names (the reference's state-dict names) as a parameter or a buffer."""
+    return set(names) <= named_tensors(module).keys()
+
+
+def wants_grad(*modules):
+    """True when autograd is recording and a parameter of the modules requires a gradient (the native front end is forward-only)."""
+    return torch.is_grad_enabled() and any(p.requires_grad for m in modules for p in m.parameters())
+
+
+def stamp(tensors, *extra):
+    """Identity of tensors at their current contents: changes when one is replaced or updated in place (optimizer steps bump
+    tensor._version)."""
+    return tuple((t.data_ptr(), t._version) for t in tensors) + extra
+
+
+def packed(module, key, names, entry, n_floats, dev, *lead):
+    """Buffer of n_floats that the library packer `entry`(*lead, tensors, n, out, stream) fills from the module's tensors
+    `names` (parameters or buffers), cached on the module under `key`.  A changed stamp re-packs into a fresh buffer, so a
+    consumer of the old one is unaffected."""
+    have = named_tensors(module)
+    lost = [n for n in names if n not in have]
+    if lost:
+        raise _lib.NeurayB200Error(f"{type(module).__name__}: tensors {lost[:3]}... not found (expected the reference's state-dict names)")
+    tensors = [have[n] for n in names]
+    st = stamp(tensors, str(dev), *lead)
+    cache = module.__dict__.setdefault("_nr_packed", {})
+    hit = cache.get(key)
+    if hit is None or hit[0] != st:
+        if tensors[0].device != torch.device(dev):
+            raise _lib.NeurayB200Error(f"{type(module).__name__}: parameters live on {tensors[0].device} but the inputs are on {dev}")
+        keep = [_lib.f32(t) for t in tensors]
+        ptrs = (C.c_void_p * len(keep))(*[t.data_ptr() for t in keep])
+        out = torch.empty(n_floats, dtype=torch.float32, device=dev)
+        _lib.call(entry, *lead, ptrs, len(keep), _lib.ptr(out), on=out)
+        hit = cache[key] = (st, out)
+    return hit[1]
 
 
 def point_index_map(params, dec, agg):
@@ -99,25 +140,22 @@ def camera_blocks(que_imgs_info=None, ref_imgs_info=None):
     """que_cam [24] and/or view_params [rfn,20] through nr_camera_blocks (one launch, no host sync)."""
     src = que_imgs_info if que_imgs_info is not None else ref_imgs_info
     dev = src["poses"].device
-    f = lambda t: t.detach().float().contiguous()
     cam = vp = None
     args = [None] * 6
     rfn = 0
     keep = []
     if que_imgs_info is not None:
-        keep += [f(que_imgs_info["poses"][0]), f(que_imgs_info["Ks"][0])]
+        keep += [_lib.f32(que_imgs_info["poses"][0]), _lib.f32(que_imgs_info["Ks"][0])]
         rng = que_imgs_info.get("depth_range")
-        keep.append(f(rng[0]) if rng is not None else None)
+        keep.append(_lib.f32(rng[0]) if rng is not None else None)
         args[0:3] = [_lib.ptr(t) for t in keep[-3:]]
         cam = torch.empty(24, dtype=torch.float32, device=dev)
     if ref_imgs_info is not None:
-        keep += [f(ref_imgs_info["poses"]), f(ref_imgs_info["Ks"])]
+        keep += [_lib.f32(ref_imgs_info["poses"]), _lib.f32(ref_imgs_info["Ks"])]
         rng = ref_imgs_info.get("depth_range")
-        keep.append(f(rng) if rng is not None else None)
+        keep.append(_lib.f32(rng) if rng is not None else None)
         args[3:6] = [_lib.ptr(t) for t in keep[-3:]]
         rfn = ref_imgs_info["poses"].shape[0]
         vp = torch.empty(rfn, 20, dtype=torch.float32, device=dev)
-    with _lib.on_device(src["poses"]):
-        _lib.check(_lib.lib().nr_camera_blocks(*args, rfn, _lib.ptr(cam), _lib.ptr(vp), _lib.stream_of(src["poses"])), "nr_camera_blocks")
-    _lib.count_launches(1)
+    _lib.call("nr_camera_blocks", *args, rfn, _lib.ptr(cam), _lib.ptr(vp), on=src["poses"])
     return cam, vp
