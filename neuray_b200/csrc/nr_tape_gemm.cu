@@ -130,15 +130,22 @@ __global__ void __launch_bounds__(256) tape_gemm_kernel(const __grid_constant__ 
         const float* za = zs + min(16 * mt + g, n_out - 1) * LDK + t4;
         const float* zb = zs + min(16 * mt + g + 8, n_out - 1) * LDK + t4;
         const float* xb = xs + min(8 * nt + g, n_in - 1) * LDK + t4;
+        // The tensor cores truncate their fp32 accumulator (about 1e-7 of the running sum per MMA, toward zero; see the
+        // conv kernel in nr_encoder.cu).  Chained over every chunk of a CTA (up to ~4 100 MMAs at the training shape) that
+        // lost 1.2e-4 of a same-sign sum (tests/test_backward_gpu.py, accuracy test).  So a chunk accumulates from zero and
+        // is added to the running sum with a rounding FADD: 1.9e-6.
+        float part[4] = {0.f, 0.f, 0.f, 0.f};
         for (int ks = kpart; ks < KC / 8; ks += ksplit) {
           const int k = 8 * ks;
           uint32_t ah[4], al[4], bh[2], bl[2];
           split(za[k], ah[0], al[0]); split(zb[k], ah[1], al[1]); split(za[k + 4], ah[2], al[2]); split(zb[k + 4], ah[3], al[3]);
           split(xb[k], bh[0], bl[0]); split(xb[k + 4], bh[1], bl[1]);
-          mma_tf32(acc[u], al, bh);
-          mma_tf32(acc[u], ah, bl);
-          mma_tf32(acc[u], ah, bh);
+          mma_tf32(part, al, bh);
+          mma_tf32(part, ah, bl);
+          mma_tf32(part, ah, bh);
         }
+#pragma unroll
+        for (int e = 0; e < 4; ++e) acc[u][e] += part[e];
       }
     }
     __syncthreads();                             // the buffer is refilled by the prefetch of the iteration after next
